@@ -55,7 +55,15 @@ def parse():
     ap.add_argument("--no-extras", action="store_true", help="skip the short runs of the other BASELINE configs")
     ap.add_argument("--no-graph", action="store_true", help="eager launches instead of one CUDA graph per step")
     ap.add_argument("--profile-json", default=None, help="write the per-kernel time table here")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (returned values; for a train step also "
+                         "the parameters and BatchNorm statistics it left) as DIR/<name>.npy, for comparing two builds")
+    args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
+    return args
 
 
 def measured_peaks():
@@ -241,6 +249,10 @@ class Bench(object):
                 self.opt_d = torch.optim.Adam(self.model_d.parameters(), lr=1e-3, betas=(0.9, 0.99), fused=True, capturable=True)
             else:
                 self.opt_d = B200Optim.FusedAdam(self.model_d.parameters(), lr=1e-3, betas=(0.9, 0.99))
+        # the seeded start that restore() returns to before every timed step
+        self.state = [t.detach() for m in (self.model, self.model_d) if m is not None
+                      for t in list(m.parameters()) + list(m.buffers())]
+        self.state0 = [t.clone() for t in self.state]
         self.host = self.make_host(rank)
         self.devbuf = {k: v.to(dev) for k, v in self.host.items()}
         self.names = [k for k in self.devbuf if not (self.model_d is None and k == "images_t")]
@@ -263,6 +275,21 @@ class Bench(object):
         if self.workload == "eval":
             del host["images_t"]
         return {k: (v.pin_memory() if pin else v) for k, v in host.items()}
+
+    def restore(self):
+        """Puts the models and optimizers back to their seeded start, in place (a captured graph reads
+        these tensors): parameters and buffers as initialised, optimizer state zeroed, which is where a
+        fresh SGD / Adam starts (no momentum, no moments, step count 0).  The adversarial training
+        amplifies the last-bit differences of the fp32 atomic reductions from step to step, so steps
+        that build on each other compute something different on every run; steps that all start here
+        compute the same up to rounding."""
+        import torch
+        with torch.no_grad():
+            torch._foreach_copy_(self.state, self.state0)
+            opt_state = [t for o in (self.opt, self.opt_d) if o is not None
+                         for st in o.state.values() for t in st.values() if torch.is_tensor(t)]
+            if opt_state:
+                torch._foreach_zero_(opt_state)
 
     def eager_step(self, buf):
         from dasemanticsegmentationaml_b200 import train as T
@@ -312,32 +339,41 @@ def sync_all(world):
     torch.cuda.synchronize()
 
 
-def time_resident(b, steps, warmup, clocks=None):
-    """Timed region 1: inputs resident in HBM.  -> (ms per step (max over ranks), launches, losses, clk, host ms)"""
+def time_resident(b, steps, warmup, clocks=None, dump_dir=None):
+    """Timed region 1: inputs resident in HBM.  -> (ms per step (max over ranks), launches, losses, clk, host ms)
+    Every step starts from the seeded state (Bench.restore, queued between the steps and outside their
+    event pairs), so with the same arguments each step computes the same every run.
+    dump_dir: rank 0 writes the last timed step's outputs there (dump_outputs)."""
     import torch
     import torch.distributed as dist
     from dasemanticsegmentationaml_b200 import _lib
     for _ in range(warmup):
+        b.restore()
         b.step(b.devbuf)
     sync_all(b.world)
     t_wall0 = time.time()
     l0 = _lib.launch_count
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
-    t_host0 = time.perf_counter()
-    for _ in range(steps):
+    events = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
+    host_s = 0.0
+    for e0, e1 in events:
+        b.restore()
+        e0.record()
+        t_host0 = time.perf_counter()
         losses = b.step(b.devbuf)
-    host_enqueue_ms = (time.perf_counter() - t_host0) * 1e3 / steps  # host time to queue one step
-    e1.record()
+        host_s += time.perf_counter() - t_host0
+        e1.record()
+    host_enqueue_ms = host_s * 1e3 / steps  # host time to queue one step
     sync_all(b.world)
     t_wall1 = time.time()
+    if dump_dir and b.rank == 0:   # before the launch count below, whose eager step moves the weights again
+        dump_outputs(b, losses, dump_dir)
     launches = _lib.launch_count - l0
     if b.graphed is not None:  # replays do not pass through the binding: count one eager step's launches
         l1 = _lib.launch_count
         b.eager_step(b.devbuf)
         torch.cuda.synchronize()
         launches = (_lib.launch_count - l1) * steps
-    ms = torch.tensor([e0.elapsed_time(e1)], device=b.dev)
+    ms = torch.tensor([sum(e0.elapsed_time(e1) for e0, e1 in events)], device=b.dev)
     if b.world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     clk = clocks.stop(t_wall0, t_wall1) if clocks else None
@@ -428,6 +464,40 @@ def weights_checksum(modules, buffers=False):
     return tot
 
 
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(b, result, out_dir):
+    """Writes what the last timed step computed as out_dir/<name>.npy: the values the step returns to its
+    caller (float32; the host-side evaluation numbers and confusion matrix as float64) and, for a train
+    step, the parameters and floating-point buffers (BatchNorm running statistics) of every model it
+    updated, each flattened to one float32 vector in parameters() / buffers() order.  Inputs and initial
+    weights are seeded, so two builds run with the same arguments can be compared file by file."""
+    import numpy as np
+    import torch
+    if b.workload == "eval":
+        st = b.eval_state
+        arrays = {"precision": np.array([st["precision"]]), "miou": np.array([st["miou"]]),
+                  "hist": st["hist"].cpu().numpy().reshape(NCLS, NCLS).astype(np.float64)}
+    else:
+        names = ("loss_seg", "loss_adv_g", "loss_d_src", "loss_d_tgt") if b.model_d is not None else ("loss",)
+        assert len(names) == len(result), (names, len(result))
+        arrays = {n: v.detach().float().reshape(1).cpu().numpy() for n, v in zip(names, result)}
+        for tag, m in (("seg", b.model), ("disc", b.model_d)):
+            if m is None:
+                continue
+            arrays[tag + "_params"] = torch.cat([p.detach().float().reshape(-1) for p in m.parameters()]).cpu().numpy()
+            bufs = [t.detach().float().reshape(-1) for t in m.buffers() if t.is_floating_point()]
+            if bufs:
+                arrays[tag + "_buffers"] = torch.cat(bufs).cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("bench.py: --dump-outputs would write %d bytes, more than %d" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for n, a in arrays.items():
+        np.save(os.path.join(out_dir, n + ".npy"), a)
+
+
 def dp_check(b):
     """Data-parallel consistency: after the timed steps every rank must hold bit-identical weights
     (same initial weights + identical averaged gradients); checked on a bit-level checksum."""
@@ -515,7 +585,7 @@ def run_b200(args):
         b.eager_step(b.devbuf)
     b.capture()
     clocks = ClockSampler(local) if rank == 0 else None
-    ms_step, launches, loss_vals, clk, host_ms = time_resident(b, steps, warmup, clocks)
+    ms_step, launches, loss_vals, clk, host_ms = time_resident(b, steps, warmup, clocks, args.dump_outputs)
     e2e_ms, h2d, d2h = time_e2e(b, steps)
     check = eval_hist_check(b) if args.workload == "eval" else dp_check(b)
 

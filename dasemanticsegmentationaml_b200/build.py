@@ -38,12 +38,15 @@ def _nvcc():
 
 
 def _digest(paths):
+    """Hash of the sources and flags with paths relative to the repository, so that a built tree that is
+    moved or copied (read-only, say) is not rebuilt."""
+    root = os.path.dirname(HERE)
     h = hashlib.sha1()
     for p in sorted(paths):
         with open(p, "rb") as f:
-            h.update(p.encode())
+            h.update(os.path.relpath(p, root).encode())
             h.update(f.read())
-    h.update(" ".join(NVCC_FLAGS + list(FAST_MATH_SOURCES)).encode())
+    h.update(" ".join(NVCC_FLAGS + list(FAST_MATH_SOURCES)).replace(root, "").encode())
     return h.hexdigest()
 
 

@@ -146,7 +146,8 @@ def test_checkpoint_helpers_round_trip(tmp_path):
     assert C.load_state(b, path) == []
     for (k, v), (_, w) in zip(a.state_dict().items(), b.state_dict().items()):
         assert torch.equal(v, w), k
-    # bare keys, wrapped target, partial overlay (BiSeNet.load_weight semantics)
+    # bare keys, wrapped target, partial overlay (BiSeNet.load_weight semantics); DataParallel moves the
+    # module to cuda:0 when a GPU is present, so the loaded values are compared on the host
     wrapped = torch.nn.DataParallel(DepthWiseSepBNFCDiscriminator(19))
     partial = {k: v for k, v in a.state_dict().items() if k.startswith("conv1_d")}
     assert partial
@@ -154,7 +155,7 @@ def test_checkpoint_helpers_round_trip(tmp_path):
     assert C.load_state(wrapped, partial, strict=False) == ["not.a.key"]
     for k, v in partial.items():
         if k != "not.a.key":
-            assert torch.equal(wrapped.module.state_dict()[k], v), k
+            assert torch.equal(wrapped.module.state_dict()[k].cpu(), v), k
 
 
 def test_input_tables_match_oracle():

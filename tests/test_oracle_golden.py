@@ -26,6 +26,18 @@ def close(a, b, rtol=2e-4, atol=2e-5):
     np.testing.assert_allclose(a, b, rtol=rtol, atol=atol)
 
 
+def disc_input(gold):
+    """The discriminator input of make_golden.py, regenerated from its seeded generator (the draw after
+    x, labels and ohem_labels) instead of stored whole, and checked against the stored sample."""
+    g = torch.Generator().manual_seed(5)
+    torch.randn(2, 3, 64, 128, generator=g)
+    torch.randint(0, 20, (2, 64, 128), generator=g)
+    torch.randint(0, 19, (2, 64, 128), generator=g)
+    p = torch.softmax(torch.randn(2, 19, 64, 128, generator=g), dim=1)
+    close(sample(p), gold["disc_in_sample"], rtol=1e-6, atol=0)
+    return p
+
+
 def test_seg_eval_forward_and_metric(gold):
     torch.set_num_threads(8)
     sd = O.make_bisenet_state(seed=11, randomize_bn=True)
@@ -71,7 +83,7 @@ def test_ohem(gold):
 @pytest.mark.parametrize("kind", ["dense", "dwsep", "dwsep_bn"])
 def test_discriminators(gold, kind):
     sd = O.clone_state(O.make_discriminator_state(kind, seed=3), requires_grad=True)
-    p = torch.from_numpy(gold["disc_in"]).requires_grad_(True)
+    p = disc_input(gold).requires_grad_(True)
     y = O.discriminator_forward(kind, sd, p, training=True)
     loss = O.bce_with_logits_const(y, 0.0)
     loss.backward()
