@@ -49,6 +49,39 @@ def gate(name, value, threshold):
     assert value > threshold, (name, value, threshold)
 
 
+# Element-wise gates of the direct kernel tests (test_norm_gpu, test_attention_gpu, test_heads_losses_gpu):
+# a kernel output against a float64 reference computed from the same bf16-rounded inputs.
+def bf16_ulp(ref):
+    """One bf16 ulp at |ref| (8 significant bits), float64."""
+    e = torch.frexp(ref.abs().clamp_min(2.0 ** -126))[1]
+    return torch.ldexp(torch.ones_like(ref, dtype=torch.float64), e - 8)
+
+
+def assert_within(name, got, want, tol, skip=None):
+    err = (got.double() - want.double()).abs()
+    ok = err <= tol
+    if skip is not None:
+        ok = ok | skip
+    worst = (err / tol).max().item() if err.numel() else 0.0
+    print("%-44s max err/tol %.3f" % (name, worst))
+    if not bool(ok.all()):
+        i = int((~ok).reshape(-1).nonzero()[0])
+        raise AssertionError("%s: %d elements out of bound; first at flat %d: got %r want %r tol %r" % (
+            name, int((~ok).sum()), i, got.reshape(-1)[i].item(), want.reshape(-1)[i].item(),
+            tol.reshape(-1)[i].item() if torch.is_tensor(tol) and tol.numel() > 1 else float(tol)))
+
+
+def assert_bf16(name, got, want, terms=None, skip=None):
+    tol = bf16_ulp(want)
+    if terms is not None:
+        tol = tol + 1e-4 * terms
+    assert_within(name, got, want, tol, skip)
+
+
+def assert_f32_sum(name, got, want, abs_terms):
+    assert_within(name, got, want, 1e-5 * abs_terms.double() + 1e-6)
+
+
 class quantised_oracle(object):
     """Context manager: oracle stores conv outputs / activations as bf16 like the CUDA path
     (SURVEY 8c quantisation-matched oracle)."""

@@ -131,6 +131,57 @@ def test_ctypes_wrappers_match_header_arity():
     assert len(seen) >= 30
 
 
+# Entry points that compute nothing a test could compare: library queries, diagnostics, the NCCL plumbing.
+NOT_COMPUTE = {"b200_version", "b200_check_device", "b200_last_error", "b200_optim_chunk",
+               "b200_debug_timeline", "b200_debug_knob", "b200_nccl_unique_id", "b200_nccl_init",
+               "b200_nccl_allreduce_grads", "b200_nccl_allreduce_hist", "b200_nccl_destroy"}
+# Entry points checked exactly through a higher-level call: entry point -> (test file, test, why that suffices).
+CHECKED_THROUGH = {
+    "b200_image_resize_normalize": ("test_input_gpu.py", "test_reference_dataset_items_bit_exact",
+                                    "bit-exact against the reference dataset items through dataset"),
+    "b200_label_resize_remap": ("test_input_gpu.py", "test_reference_dataset_items_bit_exact",
+                                "bit-exact against the reference dataset labels through dataset"),
+    "b200_count_equal": ("test_modules_gpu.py", "test_eval_metric_bit_exact",
+                         "utils.compute_global_accuracy equals the oracle's exactly"),
+    "b200_wgrad_unscratch_pairview": ("test_modules_gpu.py", "test_dense_discriminator_pair_view",
+                                      "the pair-view weight gradient is compared with torch's"),
+    "b200_upsample_fwd": ("test_modules_gpu.py", "test_fused_losses_against_torch",
+                          "every mode through losses.py against F.interpolate + torch's losses"),
+    "b200_upsample_bwd": ("test_modules_gpu.py", "test_fused_losses_against_torch",
+                          "every mode's gradient through losses.py against torch autograd"),
+    "b200_sgd_step": ("test_blocks_gpu.py", "test_fused_optimizers_match_torch",
+                      "optim.py's fused step against torch.optim.SGD"),
+    "b200_adam_step": ("test_blocks_gpu.py", "test_fused_optimizers_match_torch",
+                       "optim.py's fused step against torch.optim.Adam"),
+}
+
+
+def test_every_compute_entry_point_has_a_direct_gpu_test():
+    """Every compute entry point of include/b200seg.h is named in some tests/*_gpu.py, as its b200_ symbol or as
+    `K.<wrapper>(` of its kernels.py wrapper, or is listed above with the test that checks it -- so a new kernel
+    cannot land without a direct test."""
+    import ast
+    import glob
+    header = re.sub(r"/\*.*?\*/", "", open(os.path.join(ROOT, "include", "b200seg.h")).read(), flags=re.S)
+    names = sorted(set(re.findall(r"\b(b200_\w+)\s*\(", header)))
+    assert len(names) >= 35
+    wrappers = {}
+    tree = ast.parse(open(os.path.join(ROOT, "dasemanticsegmentationaml_b200", "kernels.py")).read())
+    for fn in tree.body:
+        if isinstance(fn, ast.FunctionDef):
+            for node in ast.walk(fn):
+                if isinstance(node, ast.Constant) and isinstance(node.value, str) and node.value.startswith("b200_"):
+                    wrappers.setdefault(node.value, set()).add(fn.name)
+    tests = {os.path.basename(p): open(p).read() for p in glob.glob(os.path.join(ROOT, "tests", "*_gpu.py"))}
+    text = "\n".join(tests.values())
+    for name, (fname, test, why) in CHECKED_THROUGH.items():
+        assert name in names, "allow-listed entry point %s is not declared" % name
+        assert "def %s(" % test in tests.get(fname, ""), "%s: %s::%s does not exist" % (name, fname, test)
+    untested = [n for n in names if n not in NOT_COMPUTE and n not in CHECKED_THROUGH and n not in text
+                and not any("K.%s(" % w in text for w in wrappers.get(n, ()))]
+    assert not untested, "entry points without a direct GPU test: %s" % untested
+
+
 def test_checkpoint_helpers_round_trip(tmp_path):
     """train.py:110,118,282-283: seg-net files carry bare keys, discriminator files `module.`-prefixed
     ones (the shipped GTA5_10_D1.pth); both must load into bare and wrapped modules."""
