@@ -10,7 +10,11 @@
 //              reverse_one_hot (argmax over classes)                    utils.py:98-122
 //              OHEM_CrossEntroy_Loss                                    utils.py:256-271
 // Low-resolution logits are fp32 NHWC with a pixel stride of `lr_ld` floats (classes padded).
+// Every kernel is a template on the class count NC; b200_upsample_fwd / _bwd pick the exact instance
+// for 2..32 classes, so the per-class loops have no masking and no padding class is ever read.
 #include <stdint.h>
+
+#include <atomic>
 
 #include "ptx.cuh"
 #include "status.h"
@@ -91,25 +95,31 @@ constexpr int LJ = 6;        // low-res columns under a 32-pixel wide tile: 31 *
 constexpr int LI_ROW = 3;    // low-res rows under 8 full-resolution rows:   7 * sh + 2 <= 3
 constexpr int SH_ROWS = 64;  // rows of a backward strip (8 warps x 8 rows)
 constexpr int LI = 11;       // low-res rows under a strip:                 63 * sh + 2 <= 11
-constexpr int kLP = 20;      // floats per staged low-res pixel (19 classes, float4 aligned)
+// Floats per staged low-res pixel: the class count rounded up to a float4 (20 for 19 classes).  The
+// staging copies exactly that many floats of each pixel, which the host check lr_ld >= round_up(NC, 4)
+// keeps inside the pixel.
+template <int NC>
+__host__ __device__ constexpr int staged_width() { return (NC + 3) / 4 * 4; }
 
-template <int ROWS>
+template <int ROWS, int NC>
 __device__ __forceinline__ void stage_lowres(const float* __restrict__ lr, int lr_ld, int h_lr, int w_lr, int n,
                                              int i_min, int j_min, float* s_lr) {
-  for (int idx = threadIdx.x; idx < ROWS * LJ * 5; idx += blockDim.x) {
-    const int q = idx % 5, pix = idx / 5, jj = pix % LJ, ii = pix / LJ;
+  constexpr int NV = staged_width<NC>() / 4;
+  for (int idx = threadIdx.x; idx < ROWS * LJ * NV; idx += blockDim.x) {
+    const int q = idx % NV, pix = idx / NV, jj = pix % LJ, ii = pix / LJ;
     const int i = min(i_min + ii, h_lr - 1), j = min(j_min + jj, w_lr - 1);
-    reinterpret_cast<float4*>(s_lr)[pix * 5 + q] =
+    reinterpret_cast<float4*>(s_lr)[pix * NV + q] =
         __ldg(reinterpret_cast<const float4*>(lr + (((int64_t)n * h_lr + i) * w_lr + j) * lr_ld) + q);
   }
 }
 template <int NC>
 __device__ __forceinline__ void sample_smem(const float* s_lr, const Interp& ih, const Interp& iw, int i_min,
                                             int j_min, float (&v)[NC]) {
-  const float4* p00 = reinterpret_cast<const float4*>(s_lr + ((ih.i0 - i_min) * LJ + iw.i0 - j_min) * kLP);
-  const float4* p01 = reinterpret_cast<const float4*>(s_lr + ((ih.i0 - i_min) * LJ + iw.i1 - j_min) * kLP);
-  const float4* p10 = reinterpret_cast<const float4*>(s_lr + ((ih.i1 - i_min) * LJ + iw.i0 - j_min) * kLP);
-  const float4* p11 = reinterpret_cast<const float4*>(s_lr + ((ih.i1 - i_min) * LJ + iw.i1 - j_min) * kLP);
+  constexpr int LP = staged_width<NC>();
+  const float4* p00 = reinterpret_cast<const float4*>(s_lr + ((ih.i0 - i_min) * LJ + iw.i0 - j_min) * LP);
+  const float4* p01 = reinterpret_cast<const float4*>(s_lr + ((ih.i0 - i_min) * LJ + iw.i1 - j_min) * LP);
+  const float4* p10 = reinterpret_cast<const float4*>(s_lr + ((ih.i1 - i_min) * LJ + iw.i0 - j_min) * LP);
+  const float4* p11 = reinterpret_cast<const float4*>(s_lr + ((ih.i1 - i_min) * LJ + iw.i1 - j_min) * LP);
   const float w00 = ih.l0 * iw.l0, w01 = ih.l0 * iw.l1, w10 = ih.l1 * iw.l0, w11 = ih.l1 * iw.l1;
   constexpr int NV = (NC + 3) / 4;
 #pragma unroll
@@ -261,7 +271,7 @@ upsample_fwd_tiled_kernel(const float* __restrict__ lr, int lr_ld, int N, int h_
                           int mode, void* __restrict__ out, int out_is_bf16_or_u8, int p_ld,
                           const int64_t* __restrict__ labels, int ignore_index,
                           double* __restrict__ acc, float* __restrict__ loss_map) {
-  __shared__ __align__(16) float s_lr[LI_ROW * LJ * kLP];
+  __shared__ __align__(16) float s_lr[LI_ROW * LJ * staged_width<NC>()];
   __shared__ Interp s_iw[TW], s_ih[TH];
   __shared__ float s_part[2][TH];
   const float sh = H > 1 ? (float)(h_lr - 1) / (float)(H - 1) : 0.f;
@@ -275,7 +285,7 @@ upsample_fwd_tiled_kernel(const float* __restrict__ lr, int lr_ld, int N, int h_
   if (threadIdx.x >= TW && threadIdx.x < TW + TH)
     s_ih[threadIdx.x - TW] = interp_at(min(h_base + threadIdx.x - TW, H - 1), sh, h_lr);
   __syncthreads();
-  stage_lowres<LI_ROW>(lr, lr_ld, h_lr, w_lr, n, s_ih[0].i0, s_iw[0].i0, s_lr);
+  stage_lowres<LI_ROW, NC>(lr, lr_ld, h_lr, w_lr, n, s_ih[0].i0, s_iw[0].i0, s_lr);
   __syncthreads();
   const int h = h_base + ty, w = w_base + tx;
   float loss = 0.f, valid = 0.f;
@@ -373,6 +383,14 @@ upsample_fwd_tiled_kernel(const float* __restrict__ lr, int lr_ld, int N, int h_
 //           pixel_weight: nullptr (all ones) or the OHEM selection weights
 //   mode 2: G = P * (dP - sum_k P_k dP_k)   with dP bf16 NHWC (stride p_ld)   (softmax)
 // One CTA = one TH x TW tile; the separable transposed interpolation runs in shared memory.
+// Per-pixel class strides of the backward kernels' shared buffers, odd so that the 32 lanes of a warp, one
+// pixel each, write one class into 32 different banks (an even stride folds them onto NC/2..1 banks: 16 classes
+// made the strip kernel 1.7x slower than 19).  19 classes keep their strides (19 and 21).
+template <int NC>
+__host__ __device__ constexpr int strip_class_stride() { return NC | 1; }
+template <int NC>
+__host__ __device__ constexpr int tile_class_stride() { return (NC + 2) | 1; }
+
 template <int NC>
 __global__ void __launch_bounds__(TH * TW)
 upsample_bwd_kernel(const float* __restrict__ lr, int lr_ld, int N, int h_lr, int w_lr, int H, int W,
@@ -381,7 +399,7 @@ upsample_bwd_kernel(const float* __restrict__ lr, int lr_ld, int N, int h_lr, in
                     const float* __restrict__ pixel_weight, const float* __restrict__ coef_num,
                     const double* __restrict__ coef_den, float coef_scale, float* __restrict__ d_lr,
                     double* __restrict__ loss_acc) {
-  __shared__ float s_g[TH][TW][NC + 2];
+  __shared__ float s_g[TH][TW][tile_class_stride<NC>()];
   __shared__ float s_loss[2][TH];
   __shared__ float s_a[TH][MAXJ][NC + 1];
   __shared__ Interp s_iw[TW], s_ih[TH];
@@ -531,6 +549,12 @@ upsample_bwd_kernel(const float* __restrict__ lr, int lr_ld, int N, int h_lr, in
 // memory).  The per-column partials are added into a CTA-wide shared buffer, reduced along w with
 // a precomputed weight table, and one atomicAdd per touched low-resolution value leaves the CTA:
 // ~1/6 of the global atomics and ~1/5 of the instructions of the generic tile kernel.
+// The staged pixels and the vertical partials live in dynamic shared memory (strip_smem_bytes: 31 KB at
+// 19 classes, 54 KB at 32, above the 48 KB of static shared memory a kernel may declare).
+template <int NC>
+constexpr int strip_smem_bytes() {
+  return (LI * LJ * staged_width<NC>() + LI * TW * strip_class_stride<NC>()) * (int)sizeof(float);
+}
 template <int NC>
 __global__ void __launch_bounds__(256)
 upsample_bwd_strip_kernel(const float* __restrict__ lr, int lr_ld, int N, int h_lr, int w_lr, int H, int W,
@@ -539,8 +563,11 @@ upsample_bwd_strip_kernel(const float* __restrict__ lr, int lr_ld, int N, int h_
                           const float* __restrict__ pixel_weight, const float* __restrict__ coef_num,
                           const double* __restrict__ coef_den, float coef_scale, float* __restrict__ d_lr,
                           double* __restrict__ loss_acc) {
-  __shared__ __align__(16) float s_lr[LI * LJ * kLP];
-  __shared__ float s_v[LI][TW][NC];   // vertical partials: [low-res row][column][class]
+  extern __shared__ __align__(16) float s_dyn[];
+  float* s_lr = s_dyn;                                   // staged low-res pixels
+  constexpr int SV = strip_class_stride<NC>();
+  float (*s_v)[TW][SV] = reinterpret_cast<float (*)[TW][SV]>(s_dyn + LI * LJ * staged_width<NC>());
+                                                         // vertical partials: [low-res row][column][class]
   __shared__ float s_wx[LJ][TW];      // weight of column x on low-res column jj
   __shared__ int s_xlo[LJ], s_xhi[LJ];
   __shared__ Interp s_iw[TW], s_ih[SH_ROWS];
@@ -555,10 +582,10 @@ upsample_bwd_strip_kernel(const float* __restrict__ lr, int lr_ld, int N, int h_
   if (threadIdx.x < TW) s_iw[threadIdx.x] = interp_at(min(w_base + threadIdx.x, W - 1), sw, w_lr);
   if (threadIdx.x >= TW && threadIdx.x < TW + SH_ROWS)
     s_ih[threadIdx.x - TW] = interp_at(min(h_base + threadIdx.x - TW, H - 1), sh, h_lr);
-  for (int i = threadIdx.x; i < LI * TW * NC; i += 256) (&s_v[0][0][0])[i] = 0.f;
+  for (int i = threadIdx.x; i < LI * TW * SV; i += 256) (&s_v[0][0][0])[i] = 0.f;
   __syncthreads();
   const int i_min = s_ih[0].i0, j_min = s_iw[0].i0;
-  if (mode != 0) stage_lowres<LI>(lr, lr_ld, h_lr, w_lr, n, i_min, j_min, s_lr);
+  if (mode != 0) stage_lowres<LI, NC>(lr, lr_ld, h_lr, w_lr, n, i_min, j_min, s_lr);
   if (threadIdx.x < LJ * TW) {  // weight table of the transposed interpolation along w
     const int jj = threadIdx.x / TW, x = threadIdx.x % TW;
     const Interp iw = s_iw[x];
@@ -627,14 +654,12 @@ upsample_bwd_strip_kernel(const float* __restrict__ lr, int lr_ld, int N, int h_
           float dp[NC];
           const __nv_bfloat16* q = static_cast<const __nv_bfloat16*>(grad_in) +
                                    (grad_is_bf16 == 2 ? padded_pixel(n, h, w, H, W) : p) * p_ld;
-          if ((p_ld & 7) == 0) {  // 16-byte aligned pixel rows: three vector loads cover 24 classes
-            uint32_t raw[12];
+          if ((p_ld & 7) == 0) {  // 16-byte aligned pixel rows: one vector load per 8 classes
+            uint32_t raw[(NC + 7) / 8 * 4];
 #pragma unroll
-            for (int k = 0; k < 3; ++k) {
-              if (8 * k < NC) {
-                const uint4 u = __ldg(reinterpret_cast<const uint4*>(q) + k);
-                raw[4 * k] = u.x; raw[4 * k + 1] = u.y; raw[4 * k + 2] = u.z; raw[4 * k + 3] = u.w;
-              }
+            for (int k = 0; k < (NC + 7) / 8; ++k) {
+              const uint4 u = __ldg(reinterpret_cast<const uint4*>(q) + k);
+              raw[4 * k] = u.x; raw[4 * k + 1] = u.y; raw[4 * k + 2] = u.z; raw[4 * k + 3] = u.w;
             }
 #pragma unroll
             for (int c = 0; c < NC; ++c) {
@@ -856,6 +881,75 @@ static int grid1d(int64_t total, int cap) {
   return (int)b;
 }
 
+static int round_up4(int v) { return (v + 3) / 4 * 4; }
+
+// Every class count with a compiled instance (kMaxCls = 32 is the widest padded logit map).
+#define B200_FOR_EACH_CLASS_COUNT(X)                                                                       \
+  X(2) X(3) X(4) X(5) X(6) X(7) X(8) X(9) X(10) X(11) X(12) X(13) X(14) X(15) X(16) X(17) X(18) X(19)      \
+  X(20) X(21) X(22) X(23) X(24) X(25) X(26) X(27) X(28) X(29) X(30) X(31) X(32)
+
+struct FwdArgs {
+  const float* lr; int lr_ld, N, h_lr, w_lr, H, W, mode; void* out; int out_flag, p_ld;
+  const int64_t* labels; int ignore_index; double* acc; float* loss_map;
+};
+struct BwdArgs {
+  const float* lr; int lr_ld, N, h_lr, w_lr, H, W, mode; const void* grad_in; int grad_is_bf16, p_ld;
+  const int64_t* labels; int ignore_index; const float* pixel_weight; const float* coef_num;
+  const double* coef_den; float coef_scale; float* d_lr; double* loss_acc;
+};
+
+template <int NC>
+static int launch_fwd(const FwdArgs& a, cudaStream_t stream) {
+  const int64_t total = (int64_t)a.N * a.H * a.W;
+  const float sh = a.H > 1 ? (float)(a.h_lr - 1) / (float)(a.H - 1) : 0.f;
+  const float sw = a.W > 1 ? (float)(a.w_lr - 1) / (float)(a.W - 1) : 0.f;
+  if (sw * (TW - 1) + 2.f <= (float)LJ && sh * (TH - 1) + 2.f <= (float)LI_ROW) {
+    const int tiles = ((a.W + TW - 1) / TW) * ((a.H + TH - 1) / TH) * a.N;
+    upsample_fwd_tiled_kernel<NC><<<tiles, TH * TW, 0, stream>>>(
+        a.lr, a.lr_ld, a.N, a.h_lr, a.w_lr, a.H, a.W, a.mode, a.out, a.out_flag, a.p_ld, a.labels, a.ignore_index,
+        a.acc, a.loss_map);
+    return check_launch("upsample_fwd(tiled)");
+  }
+  upsample_fwd_kernel<NC><<<grid1d(total, 148 * 16), 256, 0, stream>>>(
+      a.lr, a.lr_ld, a.N, a.h_lr, a.w_lr, a.H, a.W, a.mode, a.out, a.out_flag, a.p_ld, a.labels, a.ignore_index,
+      a.acc, a.loss_map);
+  return check_launch("upsample_fwd");
+}
+
+// The strip kernel's dynamic shared memory exceeds the default 48 KB limit from 28 classes on; the
+// opt-in is a per-device function attribute, set once per instance and device.
+template <int NC>
+static cudaError_t strip_smem_optin() {
+  static std::atomic<unsigned long long> done{0};
+  int dev = 0;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e != cudaSuccess) return e;
+  const unsigned long long bit = 1ull << (dev & 63);
+  if (done.load(std::memory_order_acquire) & bit) return cudaSuccess;
+  e = cudaFuncSetAttribute(upsample_bwd_strip_kernel<NC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                           strip_smem_bytes<NC>());
+  if (e == cudaSuccess) done.fetch_or(bit, std::memory_order_release);
+  return e;
+}
+
+template <int NC>
+static int launch_bwd(const BwdArgs& a, bool strip, cudaStream_t stream) {
+  if (strip) {
+    const cudaError_t e = strip_smem_optin<NC>();
+    if (e != cudaSuccess) return set_error(B200_ECUDA, "upsample_bwd(strip) shared memory: %s", cudaGetErrorString(e));
+    const int strips = ((a.W + TW - 1) / TW) * ((a.H + SH_ROWS - 1) / SH_ROWS) * a.N;
+    upsample_bwd_strip_kernel<NC><<<strips, 256, strip_smem_bytes<NC>(), stream>>>(
+        a.lr, a.lr_ld, a.N, a.h_lr, a.w_lr, a.H, a.W, a.mode, a.grad_in, a.grad_is_bf16, a.p_ld, a.labels,
+        a.ignore_index, a.pixel_weight, a.coef_num, a.coef_den, a.coef_scale, a.d_lr, a.loss_acc);
+    return check_launch("upsample_bwd(strip)");
+  }
+  const int tiles = ((a.W + TW - 1) / TW) * ((a.H + TH - 1) / TH) * a.N;
+  upsample_bwd_kernel<NC><<<tiles, TH * TW, 0, stream>>>(
+      a.lr, a.lr_ld, a.N, a.h_lr, a.w_lr, a.H, a.W, a.mode, a.grad_in, a.grad_is_bf16, a.p_ld, a.labels,
+      a.ignore_index, a.pixel_weight, a.coef_num, a.coef_den, a.coef_scale, a.d_lr, a.loss_acc);
+  return check_launch("upsample_bwd");
+}
+
 }  // namespace b200
 
 using namespace b200;
@@ -866,22 +960,20 @@ int b200_upsample_fwd(const float* lr, int lr_ld, int N, int h_lr, int w_lr, int
                       int n_classes, int mode, void* out, int out_flag, int p_ld,
                       const int64_t* labels, int ignore_index, double* acc, float* loss_map,
                       cudaStream_t stream) {
-  if (n_classes != 19) return set_error(B200_EINVAL, "upsample_fwd: only 19 classes are compiled (got %d)", n_classes);
-  if (lr_ld % 4 || lr_ld < 20) return set_error(B200_EINVAL, "upsample_fwd: logits pixel stride %d must be a multiple of 4, >= 20", lr_ld);
+  if (n_classes < 2 || n_classes > kMaxCls)
+    return set_error(B200_EINVAL, "upsample_fwd: %d classes unsupported (2..%d are compiled)", n_classes, kMaxCls);
+  if (lr_ld % 4 || lr_ld < round_up4(n_classes))
+    return set_error(B200_EINVAL, "upsample_fwd: logits pixel stride %d must be a multiple of 4, >= %d for %d classes",
+                     lr_ld, round_up4(n_classes), n_classes);
   if (mode == 2 && (p_ld % 8 || p_ld > kMaxCls || p_ld < n_classes))
     return set_error(B200_EINVAL, "upsample_fwd: probability stride %d unsupported", p_ld);
-  const int64_t total = (int64_t)N * H * W;
-  const float sh = H > 1 ? (float)(h_lr - 1) / (float)(H - 1) : 0.f;
-  const float sw = W > 1 ? (float)(w_lr - 1) / (float)(W - 1) : 0.f;
-  if (sw * (TW - 1) + 2.f <= (float)LJ && sh * (TH - 1) + 2.f <= (float)LI_ROW) {
-    const int tiles = ((W + TW - 1) / TW) * ((H + TH - 1) / TH) * N;
-    upsample_fwd_tiled_kernel<19><<<tiles, TH * TW, 0, stream>>>(
-        lr, lr_ld, N, h_lr, w_lr, H, W, mode, out, out_flag, p_ld, labels, ignore_index, acc, loss_map);
-    return check_launch("upsample_fwd(tiled)");
+  const FwdArgs a{lr, lr_ld, N, h_lr, w_lr, H, W, mode, out, out_flag, p_ld, labels, ignore_index, acc, loss_map};
+  switch (n_classes) {
+#define B200_FWD_CASE(nc) case nc: return launch_fwd<nc>(a, stream);
+    B200_FOR_EACH_CLASS_COUNT(B200_FWD_CASE)
+#undef B200_FWD_CASE
   }
-  upsample_fwd_kernel<19><<<grid1d(total, 148 * 16), 256, 0, stream>>>(
-      lr, lr_ld, N, h_lr, w_lr, H, W, mode, out, out_flag, p_ld, labels, ignore_index, acc, loss_map);
-  return check_launch("upsample_fwd");
+  return set_error(B200_EINVAL, "upsample_fwd: %d classes unsupported", n_classes);
 }
 
 int b200_upsample_bwd(const float* lr, int lr_ld, int N, int h_lr, int w_lr, int H, int W,
@@ -889,26 +981,26 @@ int b200_upsample_bwd(const float* lr, int lr_ld, int N, int h_lr, int w_lr, int
                       const int64_t* labels, int ignore_index, const float* pixel_weight,
                       const float* coef_num, const double* coef_den, float coef_scale, float* d_lr,
                       double* loss_acc, cudaStream_t stream) {
-  if (n_classes != 19) return set_error(B200_EINVAL, "upsample_bwd: only 19 classes are compiled (got %d)", n_classes);
-  if (lr_ld % 4 || lr_ld < 20) return set_error(B200_EINVAL, "upsample_bwd: logits pixel stride %d must be a multiple of 4, >= 20", lr_ld);
+  if (n_classes < 2 || n_classes > kMaxCls)
+    return set_error(B200_EINVAL, "upsample_bwd: %d classes unsupported (2..%d are compiled)", n_classes, kMaxCls);
+  if (lr_ld % 4 || lr_ld < round_up4(n_classes))
+    return set_error(B200_EINVAL, "upsample_bwd: logits pixel stride %d must be a multiple of 4, >= %d for %d classes",
+                     lr_ld, round_up4(n_classes), n_classes);
+  if (mode == 2 && p_ld < n_classes)
+    return set_error(B200_EINVAL, "upsample_bwd: probability-gradient stride %d < %d classes", p_ld, n_classes);
   const float sh = H > 1 ? (float)(h_lr - 1) / (float)(H - 1) : 0.f;
   const float sw = W > 1 ? (float)(w_lr - 1) / (float)(W - 1) : 0.f;
-  if (sw * (TW - 1) + 2.f <= (float)LJ && sh * 7.f + 2.f <= (float)LI_ROW && sh * (SH_ROWS - 1) + 2.f <= (float)LI) {
-    const int strips = ((W + TW - 1) / TW) * ((H + SH_ROWS - 1) / SH_ROWS) * N;
-    upsample_bwd_strip_kernel<19><<<strips, 256, 0, stream>>>(lr, lr_ld, N, h_lr, w_lr, H, W, mode, grad_in,
-                                                             grad_is_bf16, p_ld, labels, ignore_index,
-                                                             pixel_weight, coef_num, coef_den, coef_scale, d_lr,
-                                                             loss_acc);
-    return check_launch("upsample_bwd(strip)");
-  }
-  if (sw * (TW - 1) + 2.f > (float)MAXJ || sh * (TH - 1) + 2.f > (float)MAXI)
+  const bool strip = sw * (TW - 1) + 2.f <= (float)LJ && sh * 7.f + 2.f <= (float)LI_ROW && sh * (SH_ROWS - 1) + 2.f <= (float)LI;
+  if (!strip && (sw * (TW - 1) + 2.f > (float)MAXJ || sh * (TH - 1) + 2.f > (float)MAXI))
     return set_error(B200_EINVAL, "upsample_bwd: scale %dx%d -> %dx%d is below the supported up-sampling factor (>= 5.2 along w, >= 3.5 along h)", h_lr, w_lr, H, W);
-  const int tiles = ((W + TW - 1) / TW) * ((H + TH - 1) / TH) * N;
-  upsample_bwd_kernel<19><<<tiles, TH * TW, 0, stream>>>(lr, lr_ld, N, h_lr, w_lr, H, W, mode, grad_in,
-                                                        grad_is_bf16, p_ld, labels, ignore_index,
-                                                        pixel_weight, coef_num, coef_den, coef_scale, d_lr,
-                                                        loss_acc);
-  return check_launch("upsample_bwd");
+  const BwdArgs a{lr, lr_ld, N, h_lr, w_lr, H, W, mode, grad_in, grad_is_bf16, p_ld, labels, ignore_index,
+                  pixel_weight, coef_num, coef_den, coef_scale, d_lr, loss_acc};
+  switch (n_classes) {
+#define B200_BWD_CASE(nc) case nc: return launch_bwd<nc>(a, strip, stream);
+    B200_FOR_EACH_CLASS_COUNT(B200_BWD_CASE)
+#undef B200_BWD_CASE
+  }
+  return set_error(B200_EINVAL, "upsample_bwd: %d classes unsupported", n_classes);
 }
 
 // k-th largest (0-based rank in descending order) of `count` non-negative floats.

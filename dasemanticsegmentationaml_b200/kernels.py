@@ -26,15 +26,17 @@ def _nhwc_meta(t):
 
 
 # ------------------------------------------------------------------ filter packing
-def pack_filter(weight, transpose=False):
+def pack_filter(weight, transpose=False, rows_pad=None):
     """fp32 ``[Cout, Cin, R, S]`` -> bf16 ``[rows_pad, R*S, inner_pad]`` K-major GEMM operand.
 
     ``transpose=False``: rows = Cout (forward).  ``transpose=True``: rows = Cin (data gradient).
-    rows are padded to a multiple of 16, the inner (reduction) channel count to 32 or 64.
+    rows are padded to a multiple of 16 (or to ``rows_pad``, zero rows), the inner (reduction) channel
+    count to 32 or 64.
     """
     cout, cin, r, s = weight.shape
     rows, inner = (cin, cout) if transpose else (cout, cin)
-    rows_pad = round_up(rows, 16)
+    rows_pad = round_up(rows, 16) if rows_pad is None else rows_pad
+    assert rows_pad >= rows and rows_pad % 16 == 0
     inner_pad = round_up(inner, 32) if inner <= 32 else round_up(inner, 64)
     out = torch.empty((rows_pad, r * s, inner_pad), dtype=torch.bfloat16, device=weight.device)
     w = weight.detach()
@@ -218,10 +220,12 @@ def conv_igemm(x, filt, out, geom, bias=None, act=0, slope=0.0, stats=None, bn_t
 _wgrad_taps = {}
 
 
-def conv_wgrad(dz, x, dw, r, s, stride, pad, tune=None, scratch=None, taps=None, flops=None):
+def conv_wgrad(dz, x, dw, r, s, stride, pad, tune=None, scratch=None, taps=None, flops=None, tune_cout=None):
     """dw[Cout,Cin,R,S] (fp32) += sum_pixels dz (x) x ; dz [N,Ho,Wo,>=Cout], x [N,Hin,Win,>=Cin].
     scratch: zeroed fp32 [R*S, Cout, round_up(Cin, 16)] -- accumulate there instead (dw untouched until
-    wgrad_unscratch).  taps: explicit [(dh, dw, rs)] list of r*s taps instead of the (r, s, pad) window."""
+    wgrad_unscratch).  taps: explicit [(dh, dw, rs)] list of r*s taps instead of the (r, s, pad) window.
+    tune_cout: look the tile up under this output-channel count (the tune word sets the Cin tiling,
+    pipeline depth and pixel split only; Cout <= 128 is one row tile whatever its value)."""
     n, ho, wo, _, dz_ld = _nhwc_meta(dz)
     n2, hin, win, _, x_ld = _nhwc_meta(x)
     cout, cin = dw.shape[0], dw.shape[1]
@@ -241,7 +245,7 @@ def conv_wgrad(dz, x, dw, r, s, stride, pad, tune=None, scratch=None, taps=None,
         taps_c = _wgrad_taps[tkey] = int_array(flat)
     tap_list, taps = taps, taps_c
     if tune is None:
-        key = wgrad_key(n, ho, wo, cout, cin, r, s, stride) + ("" if tap_list is None else " v%d" % max(t[1] for t in tap_list))
+        key = wgrad_key(n, ho, wo, cout if tune_cout is None else tune_cout, cin, r, s, stride) + ("" if tap_list is None else " v%d" % max(t[1] for t in tap_list))
         tune = TUNED.get(key, 0)
         if RECORD is not None:
             RECORD.append(("wgrad", key, dict(n=n, ho=ho, wo=wo, cout=cout, cin=cin, r=r, s=s, stride=stride, pad=pad,

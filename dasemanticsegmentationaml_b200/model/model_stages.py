@@ -13,6 +13,8 @@ state_dict keys.  What changes is below the module API:
 * ``BiSeNet.forward_lowres`` exposes the 1/8- and 1/16-resolution logits so that the losses can
   fuse the bilinear up-sampling (see losses.py); ``forward`` still returns full-size logits.
 """
+import numbers
+
 import torch
 import torch.nn as nn
 
@@ -79,11 +81,30 @@ class ConvBNReLU(B200Module):
         return din, {self.conv.weight: dw, self.bn.weight: dg, self.bn.bias: db}
 
 
+# Class counts the fused up-sampling losses are compiled for (csrc/loss.cu): the logits are 32 floats per pixel.
+MIN_CLASSES, MAX_CLASSES = 2, 32
+LOGIT_CHANNELS = 32
+# The class heads' weight-gradient tiles in tuned_tiles.json were swept at 19 classes.  The tile fixes
+# the reduction (Cin) tiling and the pixel split; every count up to 32 is one output-row tile, so every
+# count uses the same entries.
+TUNED_HEAD_CLASSES = 19
+
+
+def check_n_classes(n_classes):
+    if not (isinstance(n_classes, numbers.Integral) and not isinstance(n_classes, bool)
+            and MIN_CLASSES <= n_classes <= MAX_CLASSES):
+        raise ValueError("n_classes must be an integer from %d to %d (the compiled class counts), got %r"
+                         % (MIN_CLASSES, MAX_CLASSES, n_classes))
+
+
 class BiSeNetOutput(B200Module):
     """ConvBNReLU 3x3 -> 1x1 conv to n_classes (reference model_stages.py:38-65).
-    Internally the class logits are fp32 NHWC, padded to 32 channels."""
+    Internally the class logits are fp32 NHWC, 32 channels whatever n_classes (2..32): the 1x1 filter
+    is packed as 32 rows, rows >= n_classes zero, so every class count runs the 19-class head's
+    shapes and tuned tiles."""
 
     def __init__(self, in_chan, mid_chan, n_classes, *args, **kwargs):
+        check_n_classes(n_classes)
         super(BiSeNetOutput, self).__init__()
         self.conv = ConvBNReLU(in_chan, mid_chan, ks=3, stride=1, padding=1)
         self.conv_out = nn.Conv2d(mid_chan, n_classes, kernel_size=1, bias=False)
@@ -97,7 +118,7 @@ class BiSeNetOutput(B200Module):
 
     def _fwd(self, x):
         mid, c = self.conv._fwd(x)
-        logits = ops.conv_raw_fwd(mid, self.conv_out.weight, 1, 0, out_dtype=F32)
+        logits = ops.conv_raw_fwd(mid, self.conv_out.weight, 1, 0, out_dtype=F32, rows_pad=LOGIT_CHANNELS)
         return logits, {"conv": c, "mid": mid}
 
     def _bwd(self, ctx, d_logits, need_dx=True):
@@ -106,7 +127,7 @@ class BiSeNetOutput(B200Module):
         K.cast_f32_bf16(d_logits, dz)
         mid = ctx["mid"]
         ncls = self.conv_out.weight.shape[0]
-        dw_out = ops.conv_wgrad(dz[..., :ncls], mid, self.conv_out.weight, 1, 0)
+        dw_out = ops.conv_wgrad(dz[..., :ncls], mid, self.conv_out.weight, 1, 0, tune_cout=TUNED_HEAD_CLASSES)
         d_mid = ops.conv_dgrad(dz, self.conv_out.weight, 1, 0, mid.shape[1], mid.shape[2])
         dx, g = self.conv._bwd(ctx["conv"], d_mid, None, need_dx)
         g[self.conv_out.weight] = dw_out
@@ -119,7 +140,7 @@ class BiSeNetOutput(B200Module):
 
     def _bwd_api(self, ctx, dout, need_dx=True, need_dw=True):
         n, c, h, w = dout.shape
-        d = ops.zeros_f32((n, h, w, 32), dout.device)
+        d = ops.zeros_f32((n, h, w, LOGIT_CHANNELS), dout.device)
         d[..., :c].copy_(dout.permute(0, 2, 3, 1))
         dx, g = self._bwd(ctx, d, need_dx)
         return (None if dx is None else dx.permute(0, 3, 1, 2)), g
@@ -307,6 +328,7 @@ class BiSeNet(B200Module):
 
     def __init__(self, backbone, n_classes, pretrain_model='', use_boundary_2=False, use_boundary_4=False,
                  use_boundary_8=False, use_boundary_16=False, use_conv_last=False, heat_map=False, *args, **kwargs):
+        check_n_classes(n_classes)
         super(BiSeNet, self).__init__()
         self.cp = ContextPath(backbone, pretrain_model, use_conv_last=use_conv_last)
         conv_out_inplanes = 128

@@ -17,11 +17,12 @@ F32 = torch.float32
 FORCE_REPACK = False
 
 
-def packed_filter(weight, transpose, shape=None):
+def packed_filter(weight, transpose, shape=None, rows_pad=None):
     """bf16 GEMM packing of a conv filter, cached ON the parameter object (so it dies with it and a
     recycled device address can never alias a stale packing) and refreshed when the parameter's
     version counter or storage changes (optimizer steps, load_state_dict, .to()).  ``shape``
-    reinterprets the filter memory (the stem's [32, 3, 3, 3] as a [32, 27, 1, 1] 1x1 filter)."""
+    reinterprets the filter memory (the stem's [32, 3, 3, 3] as a [32, 27, 1, 1] 1x1 filter);
+    ``rows_pad`` widens the packed rows beyond the multiple of 16 (zero rows)."""
     cache = getattr(weight, "_b200_pack", None)
     if cache is None:
         cache = {}
@@ -42,7 +43,7 @@ def packed_filter(weight, transpose, shape=None):
         K.call("b200_pack_filter", K.ptr(w), K.ptr(buf), K.c_int(cout), K.c_int(cin), K.c_int(r * s),
                K.c_int(buf.shape[0]), K.c_int(buf.shape[2]), K.c_int(int(transpose)), K.stream())
     else:
-        buf = K.pack_filter(w, transpose)
+        buf = K.pack_filter(w, transpose, rows_pad)
     cache[key] = (ver, ptr_now, buf)
     return buf
 
@@ -299,12 +300,12 @@ class ConvCtx:
 
 
 def conv_raw_fwd(x, weight, stride, pad, stats=None, bias=None, act=K.ACT_NONE, slope=0.0, out=None,
-                 out_dtype=BF16):
+                 out_dtype=BF16, rows_pad=None):
     """Implicit-GEMM convolution of an NHWC bf16 view; returns the [N,Ho,Wo,rows_pad] result."""
     n, h, w, _ = x.shape
     _, _, r, s = weight.shape
     geom = K.fwd_geometry(h, w, r, s, stride, pad)
-    filt = packed_filter(weight, False)
+    filt = packed_filter(weight, False, rows_pad=rows_pad)
     if out is None:
         out = torch.empty((n, geom.Hout, geom.Wout, filt.shape[0]), dtype=out_dtype, device=x.device)
     K.conv_igemm(x, filt, out, geom, bias=bias, act=act, slope=slope, stats=stats,
@@ -445,14 +446,15 @@ SIDE = _SideStream()
 WGRAD_SIDE_MAX_PIXELS = 65536
 
 
-def conv_wgrad(dz, x, weight, stride, pad):
+def conv_wgrad(dz, x, weight, stride, pad, tune_cout=None):
     cout, cin, r, s = weight.shape
     dw = zeros_f32((cout, cin, r, s), dz.device)
     scratch = WSCRATCH.request(dw, cout, cin, r * s)
     if WSCRATCH.depth > 0 and dz.shape[0] * dz.shape[1] * dz.shape[2] <= WGRAD_SIDE_MAX_PIXELS:
-        SIDE.run(dz.device, (dz, x, dw, scratch), lambda: K.conv_wgrad(dz, x, dw, r, s, stride, pad, scratch=scratch))
+        SIDE.run(dz.device, (dz, x, dw, scratch),
+                 lambda: K.conv_wgrad(dz, x, dw, r, s, stride, pad, scratch=scratch, tune_cout=tune_cout))
     else:
-        K.conv_wgrad(dz, x, dw, r, s, stride, pad, scratch=scratch)
+        K.conv_wgrad(dz, x, dw, r, s, stride, pad, scratch=scratch, tune_cout=tune_cout)
     return dw
 
 

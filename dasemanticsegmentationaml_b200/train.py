@@ -49,14 +49,16 @@ def allreduce_grads(params, world=None):
 
 
 def supervised_loss(model, images, labels, loss="ce", ohem_threshold=0.3567, ohem_keep=None):
-    """loss1 + loss2 + loss3 over (out, out16, out32)  (train.py:84-89 / 212-217)."""
+    """loss1 + loss2 + loss3 over (out, out16, out32)  (train.py:84-89 / 212-217), over the model's
+    ``n_classes`` classes."""
     lr = model.forward_lowres(images)
+    ncls = model.n_classes
     if loss == "ohem":
         if ohem_keep is None:
             ohem_keep = labels.numel() // 16
-        terms = [losses.upsample_ohem_cross_entropy(t, labels, ohem_threshold, ohem_keep) for t in lr]
+        terms = [losses.upsample_ohem_cross_entropy(t, labels, ohem_threshold, ohem_keep, n_classes=ncls) for t in lr]
     else:
-        terms = [losses.upsample_cross_entropy(t, labels) for t in lr]
+        terms = [losses.upsample_cross_entropy(t, labels, n_classes=ncls) for t in lr]
     return terms[0] + terms[1] + terms[2], lr
 
 
@@ -102,7 +104,7 @@ def train_da_step(model, model_D, optimizer, optimizer_D, images, labels, images
     # adversarial term on the target batch, through the frozen discriminator (train.py:223-237)
     lr_tgt = model.forward_lowres(images_t)
     optimizer.zero_grad()
-    p_tgt = losses.upsample_softmax(lr_tgt[0], H, W, zero_border=_zb(model_D))
+    p_tgt = losses.upsample_softmax(lr_tgt[0], H, W, model.n_classes, zero_border=_zb(model_D))
     d_out = model_D(p_tgt)
     loss_adv_g = losses.bce_with_logits_const(d_out, 0.0)
     (loss_adv_g * lambda_adv).backward()
@@ -113,7 +115,7 @@ def train_da_step(model, model_D, optimizer, optimizer_D, images, labels, images
     for p in model_D.parameters():
         p.requires_grad = True
     out_src = lr_src[0].detach()
-    d_out = model_D(losses.upsample_softmax(out_src, H, W, zero_border=_zb(model_D)))
+    d_out = model_D(losses.upsample_softmax(out_src, H, W, model.n_classes, zero_border=_zb(model_D)))
     loss_d_src = losses.bce_with_logits_const(d_out, 0.0)
     loss_d_src.backward()
     allreduce_grads(_opt_params(optimizer_D))
@@ -148,7 +150,7 @@ def train_da_step_nni(model, model_D, optimizer, optimizer_D, images, labels, im
     loss.backward()
 
     lr_tgt = model.forward_lowres(images_t)                         # train_nni.py:132-139
-    d_out = model_D(losses.upsample_softmax(lr_tgt[2], H, W, zero_border=_zb(model_D)))
+    d_out = model_D(losses.upsample_softmax(lr_tgt[2], H, W, model.n_classes, zero_border=_zb(model_D)))
     loss_d1 = losses.bce_with_logits_const(d_out, 0.0) * lambda_adv
     loss_d1.backward()
 
@@ -156,10 +158,10 @@ def train_da_step_nni(model, model_D, optimizer, optimizer_D, images, labels, im
         p.requires_grad = True
     out32_src = lr_src[2].detach()
     out32_tgt = lr_tgt[2].detach()
-    d_out = model_D(losses.upsample_softmax(out32_src, H, W, zero_border=_zb(model_D)))      # train_nni.py:147-151
+    d_out = model_D(losses.upsample_softmax(out32_src, H, W, model.n_classes, zero_border=_zb(model_D)))  # train_nni.py:147-151
     loss_d_src = losses.bce_with_logits_const(d_out, 0.0)
     loss_d_src.backward()
-    d_out = model_D(losses.upsample_softmax(out32_tgt, H, W, zero_border=_zb(model_D)))      # train_nni.py:153-157
+    d_out = model_D(losses.upsample_softmax(out32_tgt, H, W, model.n_classes, zero_border=_zb(model_D)))  # train_nni.py:153-157
     loss_d_tgt = losses.bce_with_logits_const(d_out, 1.0)
     loss_d_tgt.backward()
 
@@ -171,10 +173,12 @@ def train_da_step_nni(model, model_D, optimizer, optimizer_D, images, labels, im
 
 
 @torch.no_grad()
-def eval_batch(model, images, labels, n_classes=19, hist=None, pred_dtype=torch.uint8):
+def eval_batch(model, images, labels, n_classes=None, hist=None, pred_dtype=torch.uint8):
     """Forward + fused up-sample/argmax + confusion-matrix accumulation for a whole batch, all on
-    the device (train.py:30-47 handles one image at a time through the host).  Returns
-    (hist int64 [n*n] on the device, pred [N, H, W])."""
+    the device (train.py:30-47 handles one image at a time through the host).  ``n_classes`` None:
+    the model's.  Returns (hist int64 [n*n] on the device, pred [N, H, W])."""
+    if n_classes is None:
+        n_classes = model.n_classes
     model.eval()
     H, W = images.shape[2:]
     lr = model.forward_lowres(images)
@@ -196,8 +200,9 @@ def _val_batch(model, images, labels, n_classes, hist):
     return hist, correct
 
 
-def val(model, batches, n_classes=19, device=None):
-    """Evaluation loop (train.py:24-61): (mean pixel precision, mIoU).
+def val(model, batches, n_classes=None, device=None):
+    """Evaluation loop (train.py:24-61): (mean pixel precision, mIoU) over ``n_classes`` classes (None:
+    the model's).
 
     ``batches`` yields (images, labels) CUDA tensors -- this rank's shard of the evaluation set.  The
     confusion matrix and the per-image hit counts stay on the device for the whole loop (one
@@ -206,6 +211,8 @@ def val(model, batches, n_classes=19, device=None):
     images, so every rank returns the same pair.  An empty shard contributes a zero matrix.
     ``precision`` reproduces the reference's arithmetic: ``float(count) / float(total)`` per image
     (utils.py:151-159), then ``np.mean`` (train.py:56)."""
+    if n_classes is None:
+        n_classes = model.n_classes
     hist = None
     counts, totals = [], []
     for images, labels in batches:

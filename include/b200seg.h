@@ -213,6 +213,8 @@ int b200_upsum_dot_reduce(const void* dout, int dout_ld, int Ho, int Wo, const v
  * CrossEntropyLoss(ignore_index=255) (train.py:66,86-89,214-217; acc[0] += sum, acc[1] += #valid;
  * optional per-pixel loss map for OHEM), mode 2 F.softmax(dim=1) (train.py:230,248,257; bf16 NHWC out),
  * mode 3 argmax (utils.py:120-121).  lr: fp32 NHWC low-resolution logits, pixel stride lr_ld.
+ * n_classes: 2..32, each count its own compiled instance (B200_EINVAL otherwise).  lr_ld must be a
+ * multiple of 4 and >= round_up(n_classes, 4); no float of a pixel beyond round_up(n_classes, 4) is read.
  * mode 2 with out_flag == 2 (forward) / grad_is_bf16 == 2 (backward): the probability map (its gradient) is
  * the zero-bordered [N][H+2][W+2][p_ld] layout -- Conv2d's padding=1 materialised -- that the dense
  * discriminator's first layer reads as 128-byte column pairs (discriminator.py:9,18); the forward writes
