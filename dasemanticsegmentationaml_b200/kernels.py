@@ -503,6 +503,34 @@ def upsample_bwd(lr, H, W, n_classes, mode, d_lr, grad_in=None, grad_is_bf16=0, 
         tag="mode%d %dx%d" % (mode, H, W))
 
 
+def image_rescale(src, dst, mirror=False):
+    """dst = F.interpolate(src, dst.shape[2:], mode='bilinear', align_corners=True) for fp32 NCHW images;
+    mirror=True: dst holds 2N images, the second N being torch.flip of the first along the width."""
+    n, _, H, W = src.shape
+    _, _, h, w = dst.shape
+    assert src.dtype == torch.float32 and src.is_contiguous() and dst.dtype == torch.float32 and dst.is_contiguous()
+    call("b200_image_rescale", ptr(src), c_int(n), c_int(H), c_int(W), ptr(dst), c_int(h), c_int(w),
+         c_int(1 if mirror else 0), stream(), nbytes=4.0 * (src.numel() + dst.numel()), tag="%dx%d->%dx%d" % (H, W, h, w))
+    return dst
+
+
+def msc_argmax(maps, mirrored, H, W, n_classes, pred):
+    """pred [N, H, W] (uint8 or int64) = first argmax of the sum over `maps` of softmax(bilinear up-sampling to
+    H x W); maps: fp32 NHWC [N, h, w, ld] views (a mirrored half of a 2N forward is ``lr[N:]``), sampled at
+    column W-1-x where ``mirrored`` is set."""
+    n = pred.shape[0]
+    for m in maps:
+        assert m.dtype == torch.float32 and m.dim() == 4 and m.is_contiguous() and m.shape[0] == n
+    ptrs = (ctypes.c_void_p * len(maps))(*[m.data_ptr() for m in maps])
+    call("b200_msc_argmax", c_int(len(maps)), ptrs, int_array([m.shape[3] for m in maps]),
+         int_array([m.shape[1] for m in maps]), int_array([m.shape[2] for m in maps]),
+         int_array([1 if f else 0 for f in mirrored]), c_int(n), c_int(H), c_int(W), c_int(n_classes), ptr(pred),
+         c_int(1 if pred.dtype == torch.uint8 else 0), stream(),
+         nbytes=float(sum(m.numel() * 4 for m in maps) + pred.numel() * pred.element_size()),
+         tag="%d maps %dx%d" % (len(maps), H, W))
+    return pred
+
+
 def radix_select_desc(x, rank, state, hist):
     call("b200_radix_select_desc", ptr(x), c_int64(x.numel()), c_int64(rank), ptr(state), ptr(hist),
                                        stream(), nbytes=16.0 * x.numel(), tag="n%d" % x.numel())

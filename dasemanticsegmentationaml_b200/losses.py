@@ -11,6 +11,7 @@ for it.  Loss composition mirrors the reference:
 * ``bce_with_logits_const``   = BCEWithLogitsLoss against zeros / ones       (train.py:173,231-232,249-250,258)
 * ``upsample_ohem_cross_entropy`` = F.interpolate + OHEM_CrossEntroy_Loss    (utils.py:256-271)
 * ``upsample_argmax``         = F.interpolate + reverse_one_hot per sample   (utils.py:98-122)
+* ``multiscale_argmax``       = F.interpolate + softmax summed over several maps + argmax (BiSeNet's MscEval)
 """
 import torch
 
@@ -240,4 +241,16 @@ def upsample_argmax(lr, H, W, n_classes=19, dtype=torch.int64):
     out = torch.empty((n, H, W), dtype=dtype, device=lr.device)
     with torch.no_grad():
         K.upsample_fwd(lr.detach(), H, W, n_classes, K.UP_ARGMAX, out=out, out_flag=1 if dtype == torch.uint8 else 0)
+    return out
+
+
+def multiscale_argmax(maps, mirrored, H, W, n_classes=19, dtype=torch.int64):
+    """argmax over classes of sum_k softmax(upsample(maps[k])) ``[N, H, W]``, each mirrored map's up-sampled
+    probabilities flipped back along the width (BiSeNet's MscEval combine).  One unmirrored map: softmax does
+    not move the argmax, so this is ``upsample_argmax``."""
+    if len(maps) == 1 and not mirrored[0]:
+        return upsample_argmax(maps[0], H, W, n_classes, dtype)
+    out = torch.empty((maps[0].shape[0], H, W), dtype=dtype, device=maps[0].device)
+    with torch.no_grad():
+        K.msc_argmax([m.detach() for m in maps], mirrored, H, W, n_classes, out)
     return out

@@ -13,10 +13,13 @@ restated over the fused B200 ops:
   step (the reference's nn.DataParallel reduce-add, train.py:145-152,497), the evaluation
   confusion matrices are summed with an int64 all-reduce.
 """
+import math
+
 import numpy as np
 import torch
 import torch.distributed as dist
 
+from . import kernels as K
 from . import losses
 from .utils import compute_global_accuracy, fast_hist_device, per_class_iu
 
@@ -172,26 +175,83 @@ def train_da_step_nni(model, model_D, optimizer, optimizer_D, images, labels, im
     return loss.detach(), loss_d1.detach(), loss_d_src.detach(), loss_d_tgt.detach()
 
 
+MAX_TTA_MAPS = 16      # low-resolution maps one multi-scale combine takes (csrc/msc.cu)
+MAX_DENSE_BATCH = 64   # images one forward takes: the batch limit of the [N, C] dense layers
+MIN_SCALED_SIDE = 64   # smallest scaled image side predict() runs the network on
+
+
+def _tta_sizes(images, scales, flip):
+    """The scaled sizes (int(s*H), int(s*W)) of BiSeNet's MscEval, after checking the request."""
+    n, _, H, W = images.shape
+    scales = tuple(scales)
+    if not scales:
+        raise ValueError("scales must name at least one scale")
+    if any(not (math.isfinite(s) and s > 0) for s in scales):
+        raise ValueError("scales must be finite and > 0, got %r" % (scales,))
+    sizes = [(int(s * H), int(s * W)) for s in scales]
+    small = [(s, hw) for s, hw in zip(scales, sizes) if min(hw) < MIN_SCALED_SIDE]
+    if small:
+        raise ValueError("scale %r gives a %dx%d image; every scaled side must be >= %d pixels"
+                         % (small[0][0], small[0][1][0], small[0][1][1], MIN_SCALED_SIDE))
+    if len(scales) * (2 if flip else 1) > MAX_TTA_MAPS:
+        raise ValueError("%d scales%s make %d maps; at most %d are combined" % (
+            len(scales), " with flip" if flip else "", len(scales) * (2 if flip else 1), MAX_TTA_MAPS))
+    if flip and 2 * n > MAX_DENSE_BATCH:
+        raise ValueError("flip runs 2N = %d images in one forward; at most %d fit (use batches of <= %d)"
+                         % (2 * n, MAX_DENSE_BATCH, MAX_DENSE_BATCH // 2))
+    return sizes
+
+
 @torch.no_grad()
-def eval_batch(model, images, labels, n_classes=None, hist=None, pred_dtype=torch.uint8):
-    """Forward + fused up-sample/argmax + confusion-matrix accumulation for a whole batch, all on
-    the device (train.py:30-47 handles one image at a time through the host).  ``n_classes`` None:
-    the model's.  Returns (hist int64 [n*n] on the device, pred [N, H, W])."""
+def predict(model, images, n_classes=None, scales=(1.0,), flip=False, pred_dtype=torch.uint8):
+    """Class map ``[N, H, W]`` of a batch of fp32 NCHW images, optionally with BiSeNet's multi-scale + flip
+    test-time augmentation (MscEval): for each scale s the images are resized to (int(s*H), int(s*W))
+    (bilinear, align_corners=True) and, with ``flip``, mirrored along the width; the ``out`` logits of every
+    run are up-sampled to H x W (mirrored runs flipped back), their softmax probabilities summed, and the
+    first maximum taken.  One scale without flip is the argmax of the up-sampled logits; ``scales=(1.0,)``
+    without flip is exactly the single-scale evaluation of ``eval_batch``.  ``n_classes`` None: the model's."""
     if n_classes is None:
         n_classes = model.n_classes
+    if not flip and tuple(scales) == (1.0,):   # single scale: the argmax of the up-sampled logits, any image size
+        model.eval()
+        H, W = images.shape[2:]
+        return losses.upsample_argmax(model.forward_lowres(images)[0], H, W, n_classes, pred_dtype)
+    sizes = _tta_sizes(images, scales, flip)
     model.eval()
-    H, W = images.shape[2:]
-    lr = model.forward_lowres(images)
-    pred = losses.upsample_argmax(lr[0], H, W, n_classes, pred_dtype)
+    N, _, H, W = images.shape
+    maps, mirrored = [], []
+    for h, w in sizes:
+        x = images
+        if (h, w) != (H, W) or flip:
+            src = images.float().contiguous()
+            x = torch.empty((N * (2 if flip else 1), 3, h, w), dtype=torch.float32, device=images.device)
+            K.image_rescale(src, x, mirror=flip)
+        lr = model.forward_lowres(x)[0]    # a new buffer per forward: every scale's map stays valid
+        maps.append(lr[:N])
+        mirrored.append(False)
+        if flip:
+            maps.append(lr[N:])
+            mirrored.append(True)
+    return losses.multiscale_argmax(maps, mirrored, H, W, n_classes, pred_dtype)
+
+
+@torch.no_grad()
+def eval_batch(model, images, labels, n_classes=None, hist=None, pred_dtype=torch.uint8, scales=(1.0,), flip=False):
+    """Forward + fused up-sample/argmax + confusion-matrix accumulation for a whole batch, all on
+    the device (train.py:30-47 handles one image at a time through the host).  ``n_classes`` None:
+    the model's.  ``scales`` / ``flip``: multi-scale + flip evaluation, see ``predict``.
+    Returns (hist int64 [n*n] on the device, pred [N, H, W])."""
+    if n_classes is None:
+        n_classes = model.n_classes
+    pred = predict(model, images, n_classes, scales, flip, pred_dtype)
     lab = labels[:, 0] if labels.dim() == 4 else labels
     hist = fast_hist_device(lab.long(), pred, n_classes, hist)
     return hist, pred
 
 
-def _val_batch(model, images, labels, n_classes, hist):
+def _val_batch(model, images, labels, n_classes, hist, scales=(1.0,), flip=False):
     """One evaluation batch on the device -> (hist, per-image count of pred == label, int64 [N])."""
-    from . import kernels as K
-    hist, pred = eval_batch(model, images, labels, n_classes, hist)
+    hist, pred = eval_batch(model, images, labels, n_classes, hist, scales=scales, flip=flip)
     lab = labels[:, 0] if labels.dim() == 4 else labels
     if lab.dtype != torch.int64:
         lab = lab.long()
@@ -200,9 +260,9 @@ def _val_batch(model, images, labels, n_classes, hist):
     return hist, correct
 
 
-def val(model, batches, n_classes=None, device=None):
+def val(model, batches, n_classes=None, device=None, scales=(1.0,), flip=False):
     """Evaluation loop (train.py:24-61): (mean pixel precision, mIoU) over ``n_classes`` classes (None:
-    the model's).
+    the model's).  ``scales`` / ``flip``: multi-scale + flip evaluation of every batch (see ``predict``).
 
     ``batches`` yields (images, labels) CUDA tensors -- this rank's shard of the evaluation set.  The
     confusion matrix and the per-image hit counts stay on the device for the whole loop (one
@@ -215,8 +275,11 @@ def val(model, batches, n_classes=None, device=None):
         n_classes = model.n_classes
     hist = None
     counts, totals = [], []
+    # _val_batch(model, images, labels, n_classes, hist) is the per-batch seam a CPU test replaces; the
+    # multi-scale arguments are only added when they ask for more than the single-scale default
+    tta = {} if (tuple(scales), bool(flip)) == ((1.0,), False) else dict(scales=scales, flip=flip)
     for images, labels in batches:
-        hist, correct = _val_batch(model, images, labels, n_classes, hist)
+        hist, correct = _val_batch(model, images, labels, n_classes, hist, **tta)
         counts.append(correct)
         totals += [int(labels[0].numel())] * int(labels.shape[0])
         device = hist.device

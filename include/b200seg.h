@@ -245,6 +245,25 @@ int b200_bce_const_fwd(const float* x, int count, float target, float* out, cuda
 int b200_bce_const_bwd(const float* x, int count, float target, const float* gscale, float gmul,
                        float* dx, cudaStream_t stream);
 
+/* ------------------------------------------- multi-scale + flip evaluation */
+/* BiSeNet's MscEval(scales, flip) test-time augmentation.
+ * b200_image_rescale: F.interpolate(src, (h, w), mode='bilinear', align_corners=True) of fp32 NCHW images
+ * [N][3][H][W] into dst [N][3][h][w]; mirror = 1: dst is [2N][3][h][w] and images N..2N-1 are
+ * torch.flip(dst[0:N], dims=[3]), bit for bit (one forward then runs both halves: 2N <= 64, the batch
+ * limit of the network's dense layers).  h == H, w == W copies exactly.  N*h*w <= 2^30.
+ * b200_msc_argmax: pred[n][y][x] = first argmax over the n_classes classes of
+ *   sum over the maps k of softmax(up_k(y, mirrored[k] ? W-1-x : x)),
+ * up_k = bilinear align_corners=True sampling of map k (fp32 NHWC [N][h_lr[k]][w_lr[k]][lr_ld[k]], image n
+ * at maps[k] + n*h_lr*w_lr*lr_ld, so the mirrored half of a 2N forward is the same buffer offset by N images)
+ * at H x W.  1..16 maps, n_classes 2..32, lr_ld[k] a multiple of 4 and >= round_up(n_classes, 4) (as for
+ * b200_upsample_fwd), N*H*W <= 2^30.  pred: uint8 (pred_is_u8 = 1) or int64 [N][H][W].  The five arrays are
+ * host memory, copied into the kernel parameters at the call, so the call is CUDA-graph capturable. */
+int b200_image_rescale(const float* src, int N, int H, int W, float* dst, int h, int w, int mirror,
+                       cudaStream_t stream);
+int b200_msc_argmax(int n_maps, const float* const* maps, const int* lr_ld, const int* h_lr, const int* w_lr,
+                    const int* mirrored, int N, int H, int W, int n_classes, void* pred, int pred_is_u8,
+                    cudaStream_t stream);
+
 /* ------------------------------------------------- discriminator classifier */
 /* Conv2d(512, 1, 4, 2, 1) (discriminator.py:13,26,47,72,97,132): forward, data and filter gradients. */
 int b200_classifier_fwd(const void* x, int x_ld, int N, int H, int W, int C, const float* w,
