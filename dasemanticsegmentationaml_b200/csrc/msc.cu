@@ -4,7 +4,9 @@
 //                          in the same output, so that one forward runs both halves;
 //   msc_argmax_kernel<NC>  for every full-resolution pixel: bilinear (align_corners=True) sample of every
 //                          low-resolution logit map (a mirrored map at column W-1-x), softmax over the NC
-//                          classes, fp32 sum over the maps, first maximum.  Only the class map is written.
+//                          classes, fp32 sum over the maps, first maximum.  Only the class map is written;
+//   msc_confidence_kernel<NC>  the same combine, writing the class map (uint8) and the confidence of each pixel,
+//                          the mean probability of its class over the maps (pseudo-labels for self-training).
 // Compiled without --use_fast_math so that the rescale's source index and weights are PyTorch's fp32
 // arithmetic; the combine's softmax uses the __expf / __fdividef intrinsics explicitly.
 #include <stdint.h>
@@ -60,6 +62,54 @@ struct MscTable {
 
 // The map table arrives by value in the parameter block and is copied to shared memory once: indexed
 // loads from the parameter block inside the pixel loop would cost hundreds of cycles each.
+__device__ __forceinline__ void msc_stage_table(const MscTable& tab, int H, int W, MscMap* s_map, float* s_sh,
+                                                float* s_sw) {
+  if ((int)threadIdx.x < tab.n_maps) {
+    const MscMap m = tab.map[threadIdx.x];
+    s_map[threadIdx.x] = m;
+    s_sh[threadIdx.x] = H > 1 ? (float)(m.h - 1) / (float)(H - 1) : 0.f;
+    s_sw[threadIdx.x] = W > 1 ? (float)(m.w - 1) / (float)(W - 1) : 0.f;
+  }
+  __syncthreads();
+}
+
+// The per-pixel work of msc_argmax_kernel (whose own copy is kept as it was compiled before this helper
+// existed): the sum over the maps of softmax(bilinear sample at (n, y, x)) in fp32 registers, and its first
+// maximum (best, its sum bv).
+template <int NC>
+__device__ __forceinline__ void msc_accumulate(const MscMap* s_map, const float* s_sh, const float* s_sw,
+                                               int n_maps, int n, int y, int x, int W, int& best, float& bv) {
+  float acc[NC];
+#pragma unroll
+  for (int c = 0; c < NC; ++c) acc[c] = 0.f;
+  for (int k = 0; k < n_maps; ++k) {
+    const MscMap m = s_map[k];
+    const Interp ih = interp_at(y, s_sh[k], m.h), iw = interp_at(m.mirrored ? W - 1 - x : x, s_sw[k], m.w);
+    float v[NC];
+    sample_logits<NC>(m.lr, m.lr_ld, m.h, m.w, n, ih, iw, v);
+    float mx = v[0];
+#pragma unroll
+    for (int c = 1; c < NC; ++c) mx = fmaxf(mx, v[c]);
+    float s = 0.f;
+#pragma unroll
+    for (int c = 0; c < NC; ++c) {
+      v[c] = __expf(v[c] - mx);
+      s += v[c];
+    }
+    const float inv = __fdividef(1.f, s);
+#pragma unroll
+    for (int c = 0; c < NC; ++c) acc[c] += v[c] * inv;
+  }
+  best = 0;
+  bv = acc[0];
+#pragma unroll
+  for (int c = 1; c < NC; ++c)
+    if (acc[c] > bv) {
+      bv = acc[c];
+      best = c;
+    }
+}
+
 template <int NC>
 __global__ void __launch_bounds__(256)
 msc_argmax_kernel(const __grid_constant__ MscTable tab, int N, int H, int W, void* __restrict__ pred,
@@ -115,6 +165,30 @@ msc_argmax_kernel(const __grid_constant__ MscTable tab, int N, int H, int W, voi
   }
 }
 
+// The same combine, keeping the confidence of the prediction: conf = S[pred] / n_maps, the mean softmax
+// probability of the first maximum (IEEE division: msc.cu is built without --use_fast_math).
+template <int NC>
+__global__ void __launch_bounds__(256)
+msc_confidence_kernel(const __grid_constant__ MscTable tab, int N, int H, int W, uint8_t* __restrict__ pred,
+                      float* __restrict__ conf) {
+  __shared__ MscMap s_map[kMscMaxMaps];
+  __shared__ float s_sh[kMscMaxMaps], s_sw[kMscMaxMaps];
+  msc_stage_table(tab, H, W, s_map, s_sh, s_sw);
+  const int n_maps = tab.n_maps;
+  const float maps_f = (float)n_maps;
+  const int total = N * H * W;  // <= kMaxPixels (host-checked)
+  for (int p = blockIdx.x * blockDim.x + threadIdx.x; p < total; p += gridDim.x * blockDim.x) {
+    const int x = p % W;
+    const int y = (p / W) % H;
+    const int n = p / (W * H);
+    int best;
+    float bv;
+    msc_accumulate<NC>(s_map, s_sh, s_sw, n_maps, n, y, x, W, best, bv);
+    pred[p] = (uint8_t)best;
+    conf[p] = bv / maps_f;
+  }
+}
+
 static int msc_grid(int64_t total) {
   int64_t b = (total + 255) / 256;
   if (b > 148 * 16) b = 148 * 16;
@@ -124,6 +198,34 @@ static int msc_grid(int64_t total) {
 #define B200_MSC_CLASS_COUNTS(X)                                                                           \
   X(2) X(3) X(4) X(5) X(6) X(7) X(8) X(9) X(10) X(11) X(12) X(13) X(14) X(15) X(16) X(17) X(18) X(19)      \
   X(20) X(21) X(22) X(23) X(24) X(25) X(26) X(27) X(28) X(29) X(30) X(31) X(32)
+
+// The checks and the map table shared by b200_msc_argmax and b200_msc_confidence.
+static int msc_table(const char* what, int n_maps, const float* const* maps, const int* lr_ld, const int* h_lr,
+                     const int* w_lr, const int* mirrored, int N, int H, int W, int n_classes, MscTable& tab) {
+  if (n_maps < 1 || n_maps > kMscMaxMaps)
+    return set_error(B200_EINVAL, "%s: %d maps unsupported (1..%d)", what, n_maps, kMscMaxMaps);
+  if (n_classes < 2 || n_classes > kMscMaxCls)
+    return set_error(B200_EINVAL, "%s: %d classes unsupported (2..%d are compiled)", what, n_classes, kMscMaxCls);
+  if (maps == nullptr || lr_ld == nullptr || h_lr == nullptr || w_lr == nullptr || mirrored == nullptr)
+    return set_error(B200_EINVAL, "%s: NULL argument", what);
+  if (N < 1 || H < 1 || W < 1) return set_error(B200_EINVAL, "%s: sizes N=%d %dx%d must be positive", what, N, H, W);
+  const int width = (n_classes + 3) / 4 * 4;
+  tab.n_maps = n_maps;
+  for (int k = 0; k < n_maps; ++k) {
+    if (maps[k] == nullptr) return set_error(B200_EINVAL, "%s: map %d is NULL", what, k);
+    if (lr_ld[k] % 4 || lr_ld[k] < width)
+      return set_error(B200_EINVAL, "%s: map %d pixel stride %d must be a multiple of 4, >= %d for %d classes",
+                       what, k, lr_ld[k], width, n_classes);
+    if (h_lr[k] < 1 || w_lr[k] < 1)
+      return set_error(B200_EINVAL, "%s: map %d size %dx%d must be positive", what, k, h_lr[k], w_lr[k]);
+    if (mirrored[k] != 0 && mirrored[k] != 1)
+      return set_error(B200_EINVAL, "%s: map %d mirrored flag must be 0 or 1, got %d", what, k, mirrored[k]);
+    tab.map[k] = MscMap{maps[k], lr_ld[k], h_lr[k], w_lr[k], mirrored[k]};
+  }
+  if ((int64_t)N * H * W > kMaxPixels)
+    return set_error(B200_EINVAL, "%s: %d images of %dx%d exceed 2^30 pixels per launch", what, N, H, W);
+  return B200_OK;
+}
 
 }  // namespace b200
 
@@ -150,32 +252,12 @@ int b200_image_rescale(const float* src, int N, int H, int W, float* dst, int h,
 int b200_msc_argmax(int n_maps, const float* const* maps, const int* lr_ld, const int* h_lr, const int* w_lr,
                     const int* mirrored, int N, int H, int W, int n_classes, void* pred, int pred_is_u8,
                     cudaStream_t stream) {
-  if (n_maps < 1 || n_maps > kMscMaxMaps)
-    return set_error(B200_EINVAL, "msc_argmax: %d maps unsupported (1..%d)", n_maps, kMscMaxMaps);
-  if (n_classes < 2 || n_classes > kMscMaxCls)
-    return set_error(B200_EINVAL, "msc_argmax: %d classes unsupported (2..%d are compiled)", n_classes, kMscMaxCls);
-  if (maps == nullptr || lr_ld == nullptr || h_lr == nullptr || w_lr == nullptr || mirrored == nullptr ||
-      pred == nullptr)
-    return set_error(B200_EINVAL, "msc_argmax: NULL argument");
-  if (N < 1 || H < 1 || W < 1) return set_error(B200_EINVAL, "msc_argmax: sizes N=%d %dx%d must be positive", N, H, W);
+  if (pred == nullptr) return set_error(B200_EINVAL, "msc_argmax: NULL argument");
   if (pred_is_u8 != 0 && pred_is_u8 != 1)
     return set_error(B200_EINVAL, "msc_argmax: pred_is_u8 must be 0 or 1, got %d", pred_is_u8);
-  const int width = (n_classes + 3) / 4 * 4;
   MscTable tab{};
-  tab.n_maps = n_maps;
-  for (int k = 0; k < n_maps; ++k) {
-    if (maps[k] == nullptr) return set_error(B200_EINVAL, "msc_argmax: map %d is NULL", k);
-    if (lr_ld[k] % 4 || lr_ld[k] < width)
-      return set_error(B200_EINVAL, "msc_argmax: map %d pixel stride %d must be a multiple of 4, >= %d for %d classes",
-                       k, lr_ld[k], width, n_classes);
-    if (h_lr[k] < 1 || w_lr[k] < 1)
-      return set_error(B200_EINVAL, "msc_argmax: map %d size %dx%d must be positive", k, h_lr[k], w_lr[k]);
-    if (mirrored[k] != 0 && mirrored[k] != 1)
-      return set_error(B200_EINVAL, "msc_argmax: map %d mirrored flag must be 0 or 1, got %d", k, mirrored[k]);
-    tab.map[k] = MscMap{maps[k], lr_ld[k], h_lr[k], w_lr[k], mirrored[k]};
-  }
-  if ((int64_t)N * H * W > kMaxPixels)
-    return set_error(B200_EINVAL, "msc_argmax: %d images of %dx%d exceed 2^30 pixels per launch", N, H, W);
+  const int rc = msc_table("msc_argmax", n_maps, maps, lr_ld, h_lr, w_lr, mirrored, N, H, W, n_classes, tab);
+  if (rc != B200_OK) return rc;
   const int grid = msc_grid((int64_t)N * H * W);
   switch (n_classes) {
 #define B200_MSC_CASE(nc)                                                                  \
@@ -186,6 +268,25 @@ int b200_msc_argmax(int n_maps, const float* const* maps, const int* lr_ld, cons
 #undef B200_MSC_CASE
   }
   return set_error(B200_EINVAL, "msc_argmax: %d classes unsupported", n_classes);
+}
+
+int b200_msc_confidence(int n_maps, const float* const* maps, const int* lr_ld, const int* h_lr, const int* w_lr,
+                        const int* mirrored, int N, int H, int W, int n_classes, uint8_t* pred, float* conf,
+                        cudaStream_t stream) {
+  if (pred == nullptr || conf == nullptr) return set_error(B200_EINVAL, "msc_confidence: NULL argument");
+  MscTable tab{};
+  const int rc = msc_table("msc_confidence", n_maps, maps, lr_ld, h_lr, w_lr, mirrored, N, H, W, n_classes, tab);
+  if (rc != B200_OK) return rc;
+  const int grid = msc_grid((int64_t)N * H * W);
+  switch (n_classes) {
+#define B200_MSC_CASE(nc)                                                                  \
+  case nc:                                                                                 \
+    msc_confidence_kernel<nc><<<grid, 256, 0, stream>>>(tab, N, H, W, pred, conf);         \
+    return check_launch("msc_confidence");
+    B200_MSC_CLASS_COUNTS(B200_MSC_CASE)
+#undef B200_MSC_CASE
+  }
+  return set_error(B200_EINVAL, "msc_confidence: %d classes unsupported", n_classes);
 }
 
 }  // extern "C"

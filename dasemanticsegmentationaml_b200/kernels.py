@@ -531,6 +531,52 @@ def msc_argmax(maps, mirrored, H, W, n_classes, pred):
     return pred
 
 
+def msc_confidence(maps, mirrored, H, W, n_classes, pred, conf):
+    """msc_argmax writing pred uint8 [N, H, W] and conf fp32 [N, H, W] = (sum over the maps of the softmax
+    probabilities)[pred] / len(maps)."""
+    n = pred.shape[0]
+    for m in maps:
+        assert m.dtype == torch.float32 and m.dim() == 4 and m.is_contiguous() and m.shape[0] == n
+    assert pred.dtype == torch.uint8 and conf.dtype == torch.float32 and pred.shape == conf.shape == (n, H, W)
+    assert pred.is_contiguous() and conf.is_contiguous()
+    ptrs = (ctypes.c_void_p * len(maps))(*[m.data_ptr() for m in maps])
+    call("b200_msc_confidence", c_int(len(maps)), ptrs, int_array([m.shape[3] for m in maps]),
+         int_array([m.shape[1] for m in maps]), int_array([m.shape[2] for m in maps]),
+         int_array([1 if f else 0 for f in mirrored]), c_int(n), c_int(H), c_int(W), c_int(n_classes), ptr(pred),
+         ptr(conf), stream(), nbytes=float(sum(m.numel() * 4 for m in maps) + 5 * pred.numel()),
+         tag="%d maps %dx%d" % (len(maps), H, W))
+    return pred, conf
+
+
+def class_select_hist(pred, conf, n_classes, pass_, state, hist):
+    """One radix pass of the per-class selection over one batch (uint8 pred, fp32 conf, <= 2^30 pixels):
+    hist (int64 [n_classes * 256]) += the counts of the next 8 key bits, see include/b200seg.h."""
+    assert pred.dtype == torch.uint8 and conf.dtype == torch.float32 and pred.shape == conf.shape
+    assert pred.is_contiguous() and conf.is_contiguous()
+    assert state.dtype == torch.int64 and hist.dtype == torch.int64
+    call("b200_class_select_hist", ptr(pred), ptr(conf), c_int64(pred.numel()), c_int(n_classes), c_int(pass_),
+         ptr(state), ptr(hist), stream(), nbytes=5.0 * pred.numel(), tag="pass%d px%d" % (pass_, pred.numel()))
+
+
+def class_select_pick(n_classes, pass_, portion, cap, state, hist, thr, counts):
+    """Fix the next 8 bits of every class's k-th largest key; after pass 3 thr (fp32 [n]) and counts (int64 [n])."""
+    assert state.dtype == torch.int64 and hist.dtype == torch.int64
+    assert thr.dtype == torch.float32 and counts.dtype == torch.int64
+    call("b200_class_select_pick", c_int(n_classes), c_int(pass_), ctypes.c_double(portion), c_float(cap),
+         ptr(state), ptr(hist), ptr(thr), ptr(counts), stream())
+
+
+def pseudo_label_apply(pred, conf, n_classes, thr, out):
+    """out = pred where pred < n_classes and conf >= thr[pred], else 255; out uint8 (may be pred) or int64."""
+    assert pred.dtype == torch.uint8 and conf.dtype == torch.float32 and pred.shape == conf.shape == out.shape
+    assert pred.is_contiguous() and conf.is_contiguous() and out.is_contiguous()
+    assert out.dtype in (torch.uint8, torch.int64) and thr.dtype == torch.float32
+    call("b200_pseudo_label_apply", ptr(pred), ptr(conf), c_int64(pred.numel()), c_int(n_classes), ptr(thr),
+         ptr(out), c_int(1 if out.dtype == torch.uint8 else 0), stream(),
+         nbytes=float(pred.numel() * (5 + out.element_size())), tag="px%d" % pred.numel())
+    return out
+
+
 def radix_select_desc(x, rank, state, hist):
     call("b200_radix_select_desc", ptr(x), c_int64(x.numel()), c_int64(rank), ptr(state), ptr(hist),
                                        stream(), nbytes=16.0 * x.numel(), tag="n%d" % x.numel())

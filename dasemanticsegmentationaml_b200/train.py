@@ -217,6 +217,14 @@ def predict(model, images, n_classes=None, scales=(1.0,), flip=False, pred_dtype
         H, W = images.shape[2:]
         return losses.upsample_argmax(model.forward_lowres(images)[0], H, W, n_classes, pred_dtype)
     sizes = _tta_sizes(images, scales, flip)
+    maps, mirrored = _scale_maps(model, images, sizes, flip)
+    H, W = images.shape[2:]
+    return losses.multiscale_argmax(maps, mirrored, H, W, n_classes, pred_dtype)
+
+
+def _scale_maps(model, images, sizes, flip):
+    """The ``out`` low-resolution maps of MscEval's runs, one forward per scaled size (N images, or 2N with
+    their mirrors) -> (maps, mirrored flags)."""
     model.eval()
     N, _, H, W = images.shape
     maps, mirrored = [], []
@@ -232,7 +240,114 @@ def predict(model, images, n_classes=None, scales=(1.0,), flip=False, pred_dtype
         if flip:
             maps.append(lr[N:])
             mirrored.append(True)
-    return losses.multiscale_argmax(maps, mirrored, H, W, n_classes, pred_dtype)
+    return maps, mirrored
+
+
+@torch.no_grad()
+def predict_confidence(model, images, n_classes=None, scales=(1.0,), flip=False):
+    """(pred uint8 [N, H, W], conf fp32 [N, H, W]) of a batch of fp32 NCHW images: ``predict``'s class map
+    (same scales, flip and request checks) and each pixel's confidence, the mean over the runs of the softmax
+    probability of its class.  One scale without flip: the softmax of the up-sampled logits at the argmax.
+    The per-pixel input of ``pseudo_label_thresholds`` / ``pseudo_labels``.  ``n_classes`` None: the model's."""
+    if n_classes is None:
+        n_classes = model.n_classes
+    N, _, H, W = images.shape
+    # one scale without flip accepts any image size, as predict does
+    sizes = [(H, W)] if not flip and tuple(scales) == (1.0,) else _tta_sizes(images, scales, flip)
+    maps, mirrored = _scale_maps(model, images, sizes, flip)
+    pred = torch.empty((N, H, W), dtype=torch.uint8, device=images.device)
+    conf = torch.empty((N, H, W), dtype=torch.float32, device=images.device)
+    K.msc_confidence([m.detach() for m in maps], mirrored, H, W, n_classes, pred, conf)
+    return pred, conf
+
+
+MAX_SELECT_PIXELS = 1 << 30   # pixels per selection / apply launch (csrc/pseudo.cu); larger batches are split
+
+
+def _check_fraction(name, v):
+    if not (isinstance(v, (int, float)) and math.isfinite(v) and 0 < v <= 1):
+        raise ValueError("%s must be a finite number in (0, 1], got %r" % (name, v))
+
+
+def _check_classes(n_classes):
+    if not (isinstance(n_classes, int) and 2 <= n_classes <= 32):
+        raise ValueError("n_classes must be an int from 2 to 32, got %r" % (n_classes,))
+
+
+def _flat_chunks(*tensors):
+    """Views of contiguous tensors of one shape, flattened and split into runs of <= MAX_SELECT_PIXELS."""
+    flat = [t.reshape(-1) for t in tensors]
+    total = flat[0].numel()
+    for a in range(0, total, MAX_SELECT_PIXELS):
+        yield [f[a:a + MAX_SELECT_PIXELS] for f in flat]
+
+
+@torch.no_grad()
+def pseudo_label_thresholds(preds, confs, n_classes=None, portion=0.5, cap=0.9):
+    """Class-balanced pseudo-label thresholds (BDL's SSL stage, CBST): for each class c, the confidence at the
+    top ``portion`` of the pixels predicted as c, capped at ``cap``.  Exactly: with count_c the pixels of
+    class c (pred == c, conf not NaN) and k_c = min(count_c, max(1, ceil(portion * count_c))), thr_c =
+    min(k_c-th largest confidence of class c, cap) in fp32; cap for a class no pixel predicts.
+
+    ``preds`` / ``confs``: lists of per-batch tensors (uint8 / fp32 of one shape, as ``predict_confidence``
+    returns them), so a whole target set can be held at 5 bytes per pixel; they are not concatenated.  Under
+    torchrun each rank passes its shard (at least one batch) and every rank gets the thresholds of the union.
+    ``n_classes`` None: 19 (Cityscapes / GTA5).  Returns (thr fp32 [n], counts int64 [n]) on the device,
+    without a host sync."""
+    n_classes = 19 if n_classes is None else n_classes
+    _check_classes(n_classes)
+    _check_fraction("portion", portion)
+    _check_fraction("cap", cap)
+    preds, confs = list(preds), list(confs)
+    if not preds or len(preds) != len(confs):
+        raise ValueError("preds and confs must be lists of equal, non-zero length, got %d and %d"
+                         % (len(preds), len(confs)))
+    for i, (p, c) in enumerate(zip(preds, confs)):
+        if p.dtype != torch.uint8 or c.dtype != torch.float32 or p.shape != c.shape:
+            raise ValueError("batch %d: pred must be uint8 and conf fp32 of one shape, got %s %s and %s %s"
+                             % (i, p.dtype, tuple(p.shape), c.dtype, tuple(c.shape)))
+    dev = preds[0].device
+    state = torch.empty(3 * n_classes, dtype=torch.int64, device=dev)
+    hist = torch.zeros(n_classes * 256, dtype=torch.int64, device=dev)
+    thr = torch.empty(n_classes, dtype=torch.float32, device=dev)
+    counts = torch.empty(n_classes, dtype=torch.int64, device=dev)
+    batches = [(p.contiguous(), c.contiguous()) for p, c in zip(preds, confs)]
+    world = _world()
+    for pass_ in range(4):
+        for p, c in batches:
+            for fp, fc in _flat_chunks(p, c):
+                K.class_select_hist(fp, fc, n_classes, pass_, state, hist)
+        if world > 1:
+            dist.all_reduce(hist)
+        K.class_select_pick(n_classes, pass_, float(portion), float(cap), state, hist, thr, counts)
+    return thr, counts
+
+
+@torch.no_grad()
+def pseudo_labels(pred, conf, thresholds, dtype=torch.int64):
+    """Pseudo-labels [N, H, W]: pred where conf >= thresholds[pred], 255 (ignored by the losses) elsewhere and
+    where conf is NaN.  ``thresholds``: the fp32 [n] tensor of ``pseudo_label_thresholds`` (pred >= n gives
+    255), or one float, a global threshold for every class (AdaptSegNet-style SSL).  ``dtype`` int64 (for
+    ``train_step``) or uint8."""
+    if pred.dtype != torch.uint8 or conf.dtype != torch.float32 or pred.shape != conf.shape:
+        raise ValueError("pred must be uint8 and conf fp32 of one shape, got %s %s and %s %s"
+                         % (pred.dtype, tuple(pred.shape), conf.dtype, tuple(conf.shape)))
+    if dtype not in (torch.uint8, torch.int64):
+        raise ValueError("dtype must be torch.uint8 or torch.int64, got %s" % (dtype,))
+    if torch.is_tensor(thresholds):
+        if thresholds.dim() != 1 or not 2 <= thresholds.numel() <= 32:
+            raise ValueError("thresholds must be a [n] tensor with n from 2 to 32, got shape %s"
+                             % (tuple(thresholds.shape),))
+        thr = thresholds.to(device=pred.device, dtype=torch.float32).contiguous()
+    else:
+        if not (isinstance(thresholds, (int, float)) and math.isfinite(thresholds)):
+            raise ValueError("a global threshold must be a finite number, got %r" % (thresholds,))
+        thr = torch.full((32,), float(thresholds), dtype=torch.float32, device=pred.device)
+    pred, conf = pred.contiguous(), conf.contiguous()
+    out = torch.empty(pred.shape, dtype=dtype, device=pred.device)
+    for fp, fc, fo in _flat_chunks(pred, conf, out):
+        K.pseudo_label_apply(fp, fc, thr.numel(), thr, fo)
+    return out
 
 
 @torch.no_grad()

@@ -264,6 +264,37 @@ int b200_msc_argmax(int n_maps, const float* const* maps, const int* lr_ld, cons
                     const int* mirrored, int N, int H, int W, int n_classes, void* pred, int pred_is_u8,
                     cudaStream_t stream);
 
+/* ------------------------------------------- pseudo-labels for target-domain self-training */
+/* The pseudo-label round of BDL's SSL stage / CBST / IAST: predict the target set, keep each pixel's class and
+ * confidence, set a per-class threshold at the top `portion` of that class's confidences (capped), and label
+ * the pixels below it 255.  The reference writes the full-resolution logits (BiSeNet.forward,
+ * model_stages.py:241-250) and then runs softmax, max and a per-class sort in torch.
+ * b200_msc_confidence: b200_msc_argmax (same arguments and refusals) writing pred uint8 [N][H][W] and
+ *   conf fp32 [N][H][W] = S[pred] / n_maps, S the fp32 sum of the maps' softmax probabilities and pred its
+ *   first maximum.
+ * Exact per-class k-th largest confidence over any number of batches (and ranks), four 8-bit radix passes
+ * on the order-preserving key of the fp32 bit pattern (sign bit set: all bits flipped; else: sign bit set).
+ * Per pass p = 0..3: b200_class_select_hist once per batch, (with several ranks: an int64 sum of hist over
+ * them), then b200_class_select_pick once.  Pixels with pred >= n_classes or a NaN conf are not counted.
+ * b200_class_select_hist: hist[c][b] += #pixels of class c whose key matches the class's prefix found so far
+ *   (state) and whose next 8 key bits are b.  hist: uint64 [n_classes][256], zero before pass 0 (the picks
+ *   leave it zero).  count <= 2^30 pixels per call (the caller splits); state: uint64 [n_classes][3].
+ * b200_class_select_pick: one launch, no host sync; fixes the next 8 bits of each class's key and zeroes
+ *   hist.  After pass 0: count_c = #pixels of class c, k_c = min(count_c, max(1, ceil(portion * count_c)))
+ *   (float64, as Python's math.ceil).  After pass 3: thr[c] = min(k_c-th largest conf, cap) in fp32 (cap
+ *   when count_c == 0) and counts[c] = count_c (int64).  portion, cap: finite, in (0, 1].
+ * b200_pseudo_label_apply: out[i] = pred[i] if pred[i] < n_classes and conf[i] >= thr[pred[i]], else 255
+ *   (a NaN conf gives 255); out uint8 (out_is_u8 = 1, may be pred itself) or int64.  count <= 2^30. */
+int b200_msc_confidence(int n_maps, const float* const* maps, const int* lr_ld, const int* h_lr, const int* w_lr,
+                        const int* mirrored, int N, int H, int W, int n_classes, uint8_t* pred, float* conf,
+                        cudaStream_t stream);
+int b200_class_select_hist(const uint8_t* pred, const float* conf, int64_t count, int n_classes, int pass,
+                           const uint64_t* state, uint64_t* hist, cudaStream_t stream);
+int b200_class_select_pick(int n_classes, int pass, double portion, float cap, uint64_t* state, uint64_t* hist,
+                           float* thr, int64_t* counts, cudaStream_t stream);
+int b200_pseudo_label_apply(const uint8_t* pred, const float* conf, int64_t count, int n_classes, const float* thr,
+                            void* out, int out_is_u8, cudaStream_t stream);
+
 /* ------------------------------------------------- discriminator classifier */
 /* Conv2d(512, 1, 4, 2, 1) (discriminator.py:13,26,47,72,97,132): forward, data and filter gradients. */
 int b200_classifier_fwd(const void* x, int x_ld, int N, int H, int W, int C, const float* w,

@@ -6,3 +6,4 @@ python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.
 python -c "
 import json;d=json.load(open('gpurun_out/r2_bench_eval_2gpu.json'));print(d['value'],d['ms_per_step'],d['config'].get('eval_check'))"
 python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29543 scripts/check_nccl_abi.py 2>&1 | tail -3
+python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29544 scripts/check_pseudo_ranks.py 2>&1 | tail -5; echo pseudo_ranks_exit=${PIPESTATUS[0]}
