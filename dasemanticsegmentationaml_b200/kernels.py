@@ -503,6 +503,73 @@ def upsample_bwd(lr, H, W, n_classes, mode, d_lr, grad_in=None, grad_is_bf16=0, 
         tag="mode%d %dx%d" % (mode, H, W))
 
 
+# ------------------------------------------------------------------ ADVENT entropy / self-information
+ENT_SUM, ENT_MAP = 0, 1            # entropy_fwd: sum of the self-information only / also write the map
+ENT_TRAIN, ENT_SELF_INFO = 0, 1    # entropy_bwd: entropy loss + its gradient in one pass / map backward
+MAP_PLAIN, MAP_ZERO_BORDERED = 1, 2
+ENT_MAP_LD = 32                    # channels per pixel of a self-information map
+
+
+def check_entropy_args(lr, H, W, n_classes, emap=None, layout=MAP_PLAIN, others=()):
+    """The refusals of b200_entropy_fwd / _bwd, raised as ValueError before any device work."""
+    if not (isinstance(n_classes, int) and not isinstance(n_classes, bool) and 2 <= n_classes <= 32):
+        raise ValueError("n_classes must be an int from 2 to 32, got %r" % (n_classes,))
+    if not (isinstance(H, int) and isinstance(W, int) and H >= 1 and W >= 1):
+        raise ValueError("H and W must be positive ints, got %r x %r" % (H, W))
+    if lr.dim() != 4 or lr.dtype != torch.float32 or not lr.is_contiguous():
+        raise ValueError("lr must be contiguous fp32 NHWC [N, h, w, ld], got %s %s" % (lr.dtype, tuple(lr.shape)))
+    ld = lr.shape[3]
+    if ld % 4 or ld < round_up(n_classes, 4):
+        raise ValueError("logits pixel stride %d must be a multiple of 4 and >= %d for %d classes"
+                         % (ld, round_up(n_classes, 4), n_classes))
+    if emap is not None:
+        if layout not in (MAP_PLAIN, MAP_ZERO_BORDERED):
+            raise ValueError("map layout %r unknown" % (layout,))
+        if layout == MAP_ZERO_BORDERED and (H % 2 or W % 2):
+            raise ValueError("the zero-bordered layout needs even H and W, got %d x %d" % (H, W))
+        if emap.dim() != 4 or emap.shape[3] != ENT_MAP_LD:
+            raise ValueError("map pixel stride must be %d channels, got shape %s" % (ENT_MAP_LD, tuple(emap.shape)))
+        hw = (H, W) if layout == MAP_PLAIN else (H + 2, W + 2)
+        if emap.dtype != torch.bfloat16 or not emap.is_contiguous() or tuple(emap.shape[:3]) != (lr.shape[0],) + hw:
+            raise ValueError("map must be contiguous bf16 %s, got %s %s"
+                             % ((lr.shape[0],) + hw + (ENT_MAP_LD,), emap.dtype, tuple(emap.shape)))
+    for t in (lr, emap) + tuple(others):
+        if t is not None and not t.is_cuda:
+            raise ValueError("entropy kernels take CUDA tensors only, got one on %s" % (t.device,))
+
+
+def entropy_fwd(lr, H, W, n_classes, mode, emap=None, layout=MAP_PLAIN, acc=None):
+    """mode ENT_SUM: acc[0] (float64) += sum over pixels and classes of the self-information
+    I_c = -p_c log p_c / log n of p = softmax(upsample(lr)); ENT_MAP: also writes I into emap (bf16
+    [N, H, W, 32], or [N, H+2, W+2, 32] with a zero border for MAP_ZERO_BORDERED); acc may then be None."""
+    if mode not in (ENT_SUM, ENT_MAP) or (mode == ENT_SUM and acc is None) or (mode == ENT_MAP and emap is None):
+        raise ValueError("entropy_fwd: mode %r needs %s" % (mode, "acc" if mode == ENT_SUM else "a map"))
+    check_entropy_args(lr, H, W, n_classes, emap if mode == ENT_MAP else None, layout, (acc,))
+    n, h_lr, w_lr, ld = lr.shape
+    call("b200_entropy_fwd", ptr(lr), c_int(ld), c_int(n), c_int(h_lr), c_int(w_lr), c_int(H), c_int(W),
+         c_int(n_classes), c_int(mode), ptr(emap if mode == ENT_MAP else None), c_int(ENT_MAP_LD), c_int(layout),
+         ptr(acc), stream(),
+         nbytes=float(lr.numel() * 4 + (n * H * W * ENT_MAP_LD * 2 if mode == ENT_MAP else 0)),
+         tag="mode%d %dx%d" % (mode, H, W))
+
+
+def entropy_bwd(lr, H, W, n_classes, mode, d_lr, d_map=None, layout=MAP_PLAIN, acc=None):
+    """d_lr (fp32, lr's shape) += mode ENT_TRAIN: the gradient of the sum over pixels and classes of I, with
+    acc[0] += that sum (acc may be None); ENT_SELF_INFO: the gradient of sum(I * d_map) for the bf16 map
+    gradient d_map in the given layout."""
+    if mode not in (ENT_TRAIN, ENT_SELF_INFO) or (mode == ENT_SELF_INFO and d_map is None):
+        raise ValueError("entropy_bwd: mode %r needs %s" % (mode, "a map gradient" if mode == ENT_SELF_INFO else "d_lr"))
+    if d_lr.shape != lr.shape or d_lr.dtype != torch.float32 or not d_lr.is_contiguous():
+        raise ValueError("d_lr must be contiguous fp32 of lr's shape %s" % (tuple(lr.shape),))
+    check_entropy_args(lr, H, W, n_classes, d_map if mode == ENT_SELF_INFO else None, layout, (d_lr, acc))
+    n, h_lr, w_lr, ld = lr.shape
+    call("b200_entropy_bwd", ptr(lr), c_int(ld), c_int(n), c_int(h_lr), c_int(w_lr), c_int(H), c_int(W),
+         c_int(n_classes), c_int(mode), ptr(d_map if mode == ENT_SELF_INFO else None), c_int(ENT_MAP_LD),
+         c_int(layout), ptr(d_lr), ptr(acc if mode == ENT_TRAIN else None), stream(),
+         nbytes=float(lr.numel() * 8 + (n * H * W * ENT_MAP_LD * 2 if mode == ENT_SELF_INFO else 0)),
+         tag="mode%d %dx%d" % (mode, H, W))
+
+
 def image_rescale(src, dst, mirror=False):
     """dst = F.interpolate(src, dst.shape[2:], mode='bilinear', align_corners=True) for fp32 NCHW images;
     mirror=True: dst holds 2N images, the second N being torch.flip of the first along the width."""

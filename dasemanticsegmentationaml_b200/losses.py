@@ -12,6 +12,8 @@ for it.  Loss composition mirrors the reference:
 * ``upsample_ohem_cross_entropy`` = F.interpolate + OHEM_CrossEntroy_Loss    (utils.py:256-271)
 * ``upsample_argmax``         = F.interpolate + reverse_one_hot per sample   (utils.py:98-122)
 * ``multiscale_argmax``       = F.interpolate + softmax summed over several maps + argmax (BiSeNet's MscEval)
+* ``upsample_entropy``        = F.interpolate + softmax + ADVENT's entropy_loss        (csrc/entropy.cu)
+* ``upsample_self_information`` = F.interpolate + softmax + ADVENT's prob_2_entropy    (csrc/entropy.cu)
 """
 import torch
 
@@ -167,6 +169,98 @@ def upsample_softmax(lr, H, W, n_classes=19, zero_border=False):
         from .model._glue import ZeroBordered
         return _UpsampleSoftmax.apply(lr, H, W, n_classes, True).as_subclass(ZeroBordered)
     return _UpsampleSoftmax.apply(lr, H, W, n_classes, False)
+
+
+class _UpsampleEntropy(torch.autograd.Function):
+    """Training: ONE pass computes the entropy sum and the gradient of that sum w.r.t. the low-resolution
+    logits (as _UpsampleCE); backward only scales it by grad_out / (N*H*W).  Without grad: the forward-only
+    kernel."""
+
+    @staticmethod
+    def forward(ctx, lr, H, W, n_classes):
+        acc = torch.zeros(1, dtype=torch.float64, device=lr.device)
+        if ctx.needs_input_grad[0]:
+            d_lr = ops.zeros_f32(lr.shape, lr.device)
+            K.entropy_bwd(lr, H, W, n_classes, K.ENT_TRAIN, d_lr, acc=acc)
+            ctx.save_for_backward(d_lr)
+        else:
+            K.entropy_fwd(lr, H, W, n_classes, K.ENT_SUM, acc=acc)
+        count = lr.shape[0] * H * W
+        ctx.grad_mul = 1.0 / count
+        return (acc[0] / count).to(F32)
+
+    @staticmethod
+    def backward(ctx, g):
+        (d_unscaled,) = ctx.saved_tensors
+        d_lr = torch.empty_like(d_unscaled)
+        K.scale_f32(d_unscaled, g.to(F32).contiguous(), None, ctx.grad_mul, d_lr)
+        return d_lr, None, None, None
+
+
+def upsample_entropy(lr, H, W, n_classes=19):
+    """ADVENT's entropy loss (``entropy_loss(softmax(interp(pred)))``): the mean over the N x H x W pixels of
+    the normalised entropy sum_c -p_c log p_c / log n_classes of p = softmax(upsample(lr)), an fp32 scalar.
+    Nothing of size N x n x H x W is written.  Under torchrun this is the rank-local mean; the gradient average
+    of ``train.allreduce_grads`` then yields the gradient of the global mean when every rank has the same batch
+    shape (as ``train.train_minent_step`` is used), so no collective is needed here."""
+    K.check_entropy_args(lr, H, W, n_classes)
+    return _UpsampleEntropy.apply(lr, H, W, n_classes)
+
+
+def _map32(d):
+    """A logical bf16 [N, C, H, W] gradient as the [N, H, W, 32] NHWC buffer the self-information backward reads:
+    the tensor's own storage when it is laid out so, else a copy (its channels >= C are never read)."""
+    n, c, h, w = d.shape
+    v = d.detach().as_subclass(torch.Tensor).permute(0, 2, 3, 1)
+    if (v.dtype == BF16 and v.stride() == (h * w * 32, w * 32, 32, 1) and v.data_ptr() % 16 == 0
+            and v.storage_offset() + n * h * w * 32 <= v.untyped_storage().nbytes() // 2):
+        return torch.Tensor.as_strided(v, (n, h, w, 32), (h * w * 32, w * 32, 32, 1))
+    buf = torch.zeros((n, h, w, 32), dtype=BF16, device=d.device)
+    buf[..., :c].copy_(v)
+    return buf
+
+
+class _UpsampleSelfInformation(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, lr, H, W, n_classes, zero_border):
+        n = lr.shape[0]
+        if zero_border:
+            # [N, H+2, W+2, 32] with the map at rows / cols 1..H / 1..W; the kernel writes the zero border
+            m = torch.empty((n, H + 2, W + 2, 32), dtype=BF16, device=lr.device)
+            K.entropy_fwd(lr, H, W, n_classes, K.ENT_MAP, emap=m, layout=K.MAP_ZERO_BORDERED)
+            m = m[:, 1:H + 1, 1:W + 1]
+        else:
+            m = torch.empty((n, H, W, 32), dtype=BF16, device=lr.device)
+            K.entropy_fwd(lr, H, W, n_classes, K.ENT_MAP, emap=m, layout=K.MAP_PLAIN)
+        ctx.save_for_backward(lr)
+        ctx.meta = (H, W, n_classes)
+        return m.permute(0, 3, 1, 2)[:, :n_classes]
+
+    @staticmethod
+    def backward(ctx, dm):
+        (lr,) = ctx.saved_tensors
+        H, W, n_classes = ctx.meta
+        from .model._glue import padded_base, padded_strides
+        d_lr = ops.zeros_f32(lr.shape, lr.device)
+        if padded_strides(dm):   # the dense discriminator's pair-view data gradient: read it where it lies
+            K.entropy_bwd(lr, H, W, n_classes, K.ENT_SELF_INFO, d_lr, d_map=padded_base(dm),
+                          layout=K.MAP_ZERO_BORDERED)
+        else:
+            K.entropy_bwd(lr, H, W, n_classes, K.ENT_SELF_INFO, d_lr, d_map=_map32(dm), layout=K.MAP_PLAIN)
+        return d_lr, None, None, None, None
+
+
+def upsample_self_information(lr, H, W, n_classes=19, zero_border=False):
+    """ADVENT's self-information map (``prob_2_entropy(softmax(interp(pred)))``): -p_c log p_c / log n_classes
+    of p = softmax(upsample(lr)) as a bf16 channels-last ``[N, n_classes, H, W]`` view of a 32-channel NHWC
+    buffer whose padding channels are zero -- the AdvEnt discriminator's input.  zero_border=True with even H
+    and W: a ``ZeroBordered`` view of the interior of an [N, H+2, W+2, 32] buffer with a zero border, which
+    ``FCDiscriminator`` reads as column pairs; otherwise a plain view (exactly as ``upsample_softmax``)."""
+    K.check_entropy_args(lr, H, W, n_classes)
+    if zero_border and H % 2 == 0 and W % 2 == 0:
+        from .model._glue import ZeroBordered
+        return _UpsampleSelfInformation.apply(lr, H, W, n_classes, True).as_subclass(ZeroBordered)
+    return _UpsampleSelfInformation.apply(lr, H, W, n_classes, False)
 
 
 class _BCEConst(torch.autograd.Function):

@@ -175,6 +175,73 @@ def train_da_step_nni(model, model_D, optimizer, optimizer_D, images, labels, im
     return loss.detach(), loss_d1.detach(), loss_d_src.detach(), loss_d_tgt.detach()
 
 
+def train_minent_step(model, optimizer, images, labels, images_t, lambda_ent=0.001):
+    """One iteration of ADVENT's MinEnt (Vu et al., CVPR 2019): the supervised loss on the labelled source
+    batch plus ``lambda_ent`` times the entropy of the target predictions (``losses.upsample_entropy`` of the
+    ``out`` logits at the target image size); gradients accumulate and the optimizer steps once.
+
+    The segmentation loss is this project's three-head ``supervised_loss`` (train.py's composition), not
+    ADVENT's DeepLab main + 0.1 * aux loss; only the target term and the step structure come from ADVENT.
+    Returns (loss_seg, loss_ent) as device scalars, without a host sync."""
+    Ht, Wt = images_t.shape[2:]
+    model.train()
+    optimizer.zero_grad()
+    loss, _ = supervised_loss(model, images, labels)
+    loss.backward()
+    lr_t = model.forward_lowres(images_t)
+    loss_ent = losses.upsample_entropy(lr_t[0], Ht, Wt, model.n_classes)
+    (lambda_ent * loss_ent).backward()
+    allreduce_grads(_opt_params(optimizer))
+    optimizer.step()
+    return loss.detach(), loss_ent.detach()
+
+
+def train_advent_step(model, model_D, optimizer, optimizer_D, images, labels, images_t, lambda_adv=0.001):
+    """One iteration of ADVENT's AdvEnt (the ``train_advent`` loop): the discriminator works on self-information
+    maps (``losses.upsample_self_information`` of the ``out`` logits) instead of on the softmax.  The net is
+    trained on the source loss plus ``lambda_adv`` times the adversarial term (target maps labelled as source,
+    through the frozen discriminator); the discriminator then learns source maps as 0 and target maps as 1,
+    each loss halved.  Gradients accumulate and each optimizer steps once, at the end.  The target map is
+    reused, detached, for the discriminator, as ``train_da_step`` reuses its softmax.
+
+    The segmentation loss is this project's three-head ``supervised_loss`` (train.py's composition), not
+    ADVENT's DeepLab main + 0.1 * aux loss, and only the main output feeds the discriminator; the target terms
+    and the step structure come from ADVENT.  Works with all three discriminators.
+    Returns (loss_seg, loss_adv, loss_d_src, loss_d_tgt), the last two halved, as device scalars."""
+    H, W = images.shape[2:]
+    Ht, Wt = images_t.shape[2:]
+    ncls = model.n_classes
+    zb = _zb(model_D)
+    optimizer.zero_grad()
+    optimizer_D.zero_grad()
+    model.train()
+    model_D.train()
+    for p in model_D.parameters():
+        p.requires_grad = False
+
+    loss, lr_src = supervised_loss(model, images, labels)
+    loss.backward()
+
+    lr_t = model.forward_lowres(images_t)
+    i_t = losses.upsample_self_information(lr_t[0], Ht, Wt, ncls, zero_border=zb)
+    loss_adv = losses.bce_with_logits_const(model_D(i_t), 0.0)
+    (lambda_adv * loss_adv).backward()
+
+    for p in model_D.parameters():
+        p.requires_grad = True
+    i_s = losses.upsample_self_information(lr_src[0].detach(), H, W, ncls, zero_border=zb)
+    loss_d_src = losses.bce_with_logits_const(model_D(i_s), 0.0) / 2
+    loss_d_src.backward()
+    loss_d_tgt = losses.bce_with_logits_const(model_D(i_t.detach()), 1.0) / 2
+    loss_d_tgt.backward()
+
+    allreduce_grads(_opt_params(optimizer))
+    allreduce_grads(_opt_params(optimizer_D))
+    optimizer.step()
+    optimizer_D.step()
+    return loss.detach(), loss_adv.detach(), loss_d_src.detach(), loss_d_tgt.detach()
+
+
 MAX_TTA_MAPS = 16      # low-resolution maps one multi-scale combine takes (csrc/msc.cu)
 MAX_DENSE_BATCH = 64   # images one forward takes: the batch limit of the [N, C] dense layers
 MIN_SCALED_SIDE = 64   # smallest scaled image side predict() runs the network on

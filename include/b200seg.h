@@ -245,6 +245,32 @@ int b200_bce_const_fwd(const float* x, int count, float target, float* out, cuda
 int b200_bce_const_bwd(const float* x, int count, float target, const float* gscale, float gmul,
                        float* dx, cudaStream_t stream);
 
+/* ------------------------------------------- ADVENT: entropy and self-information maps */
+/* ADVENT (Vu et al., CVPR 2019) on p = softmax(up(lr)), up = the bilinear align_corners=True up-sampling of
+ * b200_upsample_fwd, over the n_classes valid classes:
+ *   self-information map (prob_2_entropy)  I_c = -p_c * log(p_c) / log(n_classes)
+ *   entropy loss (entropy_loss)            E   = sum over pixels and classes of I_c / (N*H*W)
+ * p_c * log(p_c) is computed as p_c * log_softmax_c, so an fp32 probability that underflows gives 0, not NaN.
+ * lr: fp32 NHWC [N][h_lr][w_lr][lr_ld]; n_classes 2..32 (one compiled instance each); lr_ld a multiple of 4 and
+ * >= round_up(n_classes, 4) (no float of a pixel beyond that is read).  Up-sampling factor >= 7.75 along w and
+ * >= 7 along h (BiSeNet's `out` head is 1/8 of the image); N*(H+2)*(W+2) <= 2^31 - 1.
+ * The map (mode 1): bf16, p_ld == 32 channels per pixel, channels >= n_classes zero; layout 1 = [N][H][W][32],
+ * layout 2 = [N][H+2][W+2][32] with the map at rows / cols 1..H / 1..W and a zero border (the layout of
+ * b200_upsample_fwd mode 2 with out_flag 2, which the dense discriminator reads as column pairs); layout 2
+ * needs even H and W.  Every refusal returns B200_EINVAL before any device work.
+ * b200_entropy_fwd: mode 0: acc[0] += sum over pixels and classes of I (no map; acc required);
+ *   mode 1: also writes the map (the border too in layout 2); acc may be NULL.
+ * b200_entropy_bwd: both modes add into d_lr (fp32, stride lr_ld; its padding classes are not touched).
+ *   mode 0 (training pass of the entropy loss): d_lr += d(sum over pixels and classes of I)/d lr and, when acc
+ *   is not NULL, acc[0] += that sum, in one pass; b200_scale_f32 then applies grad_out / (N*H*W).
+ *   mode 1 (self-information backward): d_lr += the gradient of sum(I * dI) for the bf16 map gradient d_map
+ *   in the given layout (layout 2: only the interior is read); acc is not used. */
+int b200_entropy_fwd(const float* lr, int lr_ld, int N, int h_lr, int w_lr, int H, int W, int n_classes,
+                     int mode, void* map, int p_ld, int layout, double* acc, cudaStream_t stream);
+int b200_entropy_bwd(const float* lr, int lr_ld, int N, int h_lr, int w_lr, int H, int W, int n_classes,
+                     int mode, const void* d_map, int p_ld, int layout, float* d_lr, double* acc,
+                     cudaStream_t stream);
+
 /* ------------------------------------------- multi-scale + flip evaluation */
 /* BiSeNet's MscEval(scales, flip) test-time augmentation.
  * b200_image_rescale: F.interpolate(src, (h, w), mode='bilinear', align_corners=True) of fp32 NCHW images
